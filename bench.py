@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path on BASELINE.json's headline config.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] -- PPO, synthetic 64-dim observations, 1024 actors x
 horizon 128 (n_step = stride = 128), 2x256 MLP actor + critic, clip mode, z-filter on, A = 8.
@@ -179,10 +179,15 @@ def run_ours(args):
     from surreal_b200.replay import FIFOReplay
     from surreal_b200.distributed import LocalHub
     _lib.lib()
+    import numpy as np
     lc, ec, sc = build_configs(N_ACTORS, HORIZON)
     ec.seed = rank
+    torch.manual_seed(0)                                          # initial actor / critic weights
     la = SurrealDefaultLauncher(PPOAgent, PPOLearner, FIFOReplay, sc, ec, lc)
     agent, replay, learner = la.setup_engine()
+    # the launcher draws the actors' exploration scales from a clock-seeded generator (as the reference does); fix them
+    # so that every run with the same arguments sees the same inputs
+    agent.set_noise(np.random.default_rng(rank).uniform(-agent.log_sig_range, agent.log_sig_range, agent.num_envs))
     if world > 1:
         learner.enable_data_parallel(dist.group.WORLD)
     N, T, D, A = N_ACTORS, HORIZON, OBS_DIM, ACT_DIM
@@ -238,6 +243,8 @@ def run_ours(args):
     env_steps = N * T * args.steps * world
     value = env_steps / (total_ms / 1e3)
     opt_steps = sum(learner.epoch_history[-args.steps:]) if hasattr(learner, 'epoch_history') else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, replay, learner)
     # the two halves of a step in isolation (graph-replayed, sequential, device-timed): explains the pipelined number
     phase = {'rollout': [], 'learn': []}
     for _ in range(5):
@@ -386,6 +393,43 @@ def run_ours(args):
         sys.stdout.flush()
         sys.stderr.flush()
         os._exit(0)
+
+
+DUMP_WINDOWS = 128        # windows per batch-shaped array written by --dump-outputs (a fixed, seeded sample)
+
+
+def dump_outputs(out_dir, replay, learner):
+    """What the last timed step computed, as ``out_dir/<name>.npy`` (float64 statistics, float32 arrays; 12 MB at cfg2, 24 at cfg5):
+      stats_*   : the statistics learn() returned;
+      *_params  : the learner's parameters after the step (the actor vector ends with log_var), z_stats its z-filter;
+      batch_*   : the windows learn() consumed, with the advantages and returns it computed for them;
+      replay_*  : the windows the actors left in the replay for the next learn() (none in --sequential mode).
+    Batch-shaped arrays hold the same fixed sample of DUMP_WINDOWS window indices."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    os.makedirs(out_dir, exist_ok=True)
+    out = {'stats_' + k.lstrip('_'): np.float64(v) for k, v in learner.tensorplex.last.items()}
+    m = learner.model
+    out.update(actor_params=m.actor.params, critic_params=m.critic.params, z_stats=m.z_stats)
+    B = learner.batch_size
+    pick = np.sort(np.random.default_rng(0).choice(B, min(B, DUMP_WINDOWS), replace=False))
+    rows = torch.as_tensor(pick, device=learner.device)
+    for k, t in learner.replay_out_buffers().items():
+        out['batch_' + k] = t[rows]
+    out['batch_advantages'], out['batch_returns'] = learner._adv[rows], learner._ret[rows]
+    st = replay._read_state()
+    if st['count']:
+        slots = (st['head'] + rows[rows < st['count']]) % st['capacity']
+        for k, t in (('obs_full', replay.r_obs), ('actions', replay.r_act), ('pd', replay.r_pd),
+                     ('rewards', replay.r_rew), ('dones', replay.r_done)):
+            out['replay_' + k] = t[slots]
+    for k, v in out.items():
+        if v is None:
+            continue
+        if isinstance(v, torch.Tensor):
+            v = v.detach().float().cpu().numpy()
+        np.save(os.path.join(out_dir, k + '.npy'), v)
 
 
 def run_extras(dev, peaks, flush):
@@ -866,7 +910,13 @@ if __name__ == '__main__':
     ap.add_argument('--workload', type=str, default='cfg2', choices=['cfg2', 'cfg5'],
                     help='cfg2: BASELINE configs[1] (the metric; weak scaling).  cfg5: configs[4], 4096 actors x horizon 256 in total, '
                          'sharded over the ranks (strong scaling; use with --lite)')
+    ap.add_argument('--dump-outputs', type=str, default=None, metavar='DIR',
+                    help='after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)')
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
+    if a.dump_outputs and a.impl != 'ours':
+        ap.error('--dump-outputs writes the outputs of --impl ours')
     if a.workload == 'cfg5':
         WORKLOAD = 'cfg5'
         N_ACTORS, HORIZON = 4096 // int(os.environ.get('WORLD_SIZE', 1)), 256
