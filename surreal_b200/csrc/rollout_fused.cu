@@ -6,20 +6,26 @@
 // independent of one another, so the loop over time can move INSIDE the kernel:
 //   * a thread-block cluster of 4 CTAs owns 32 actors for the whole chunk;
 //   * each CTA keeps a QUARTER of every hidden layer's weights resident in shared memory for all T steps (fetched
-//     once with cp.async) and computes that quarter of the layer's columns for the cluster's 32 rows (fp32 FFMA,
-//     thread = 1 row x 4 columns); layer outputs are exchanged through distributed shared memory (16-byte
-//     st.shared::cluster pushes into all four copies) with one cluster barrier per layer;
-//   * each CTA then finishes ITS 8 actors: head, sampling, environment step, window staging -- one warp per actor,
-//     observations / env state never leave shared memory between steps;
+//     once with cp.async) and computes that quarter of the layer's columns for the cluster's 32 rows (fp32, packed
+//     fma.rn.f32x2); layer outputs reach the CTAs that need them through distributed shared memory;
+//   * WARP SPECIALISATION: warps 0..7 ("math warps") run the two hidden layers while warps 8..15 ("env warps") do the
+//     half of the SAME env step that does not depend on the action (Philox + Box-Muller draws, Ws.s, |s|^2) -- it
+//     depends only on the state at the top of the step, so it stays off the serial chain;
+//   * the three exchanges of a step (hidden layer 1 to all peers, last hidden layer rows to their owner, next input
+//     tile to all peers) are st.async stores that signal the consumer's mbarrier, not cluster barriers; the cyclic data
+//     dependence of a step makes "buffer free" signals unnecessary;
+//   * the head runs on all 16 warps (k slices of the last hidden layer for all 8 owned actors); then each CTA finishes
+//     ITS 8 actors -- sampling, environment step, window staging -- one warp per actor; observations / env state never
+//     leave shared memory between steps;
 //   * finished windows go to a per-actor outbox with their completion step; sb200_ppo_rollout_commit_f32 assigns
 //     FIFO slots in the reference's (step, actor) arrival order afterwards and copies them into the replay ring.
+// The schedule follows clock64 traces of the kernel (tools/rollout_trace.py, profiles/r02b_rollout_trace_*).
 // Sampling and environment arithmetic (and their Philox keys) are those of rollout.cu, so both paths draw the
-// same noise; the policy forward is fp32 FFMA (the per-step path uses 3xTF32 tensor-core products; both are
+// same noise; the policy forward is fp32 FMA (the per-step path uses 3xTF32 tensor-core products; both are
 // fp32-accurate, they differ by rounding order only).
 #include <cooperative_groups.h>
 
 #include <algorithm>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "rollout_dev.cuh"
@@ -31,7 +37,7 @@ namespace cg = cooperative_groups;
 constexpr int RF_CS = 4;            // CTAs per cluster
 constexpr int RF_ROWS = 32;         // actors per cluster
 constexpr int RF_OWN = RF_ROWS / RF_CS;
-constexpr int RF_THREADS = 512;     // 16 warps: thread (ty = row 0..31, tx = column quad 0..15)
+constexpr int RF_THREADS = 512;     // 16 warps: 8 math warps, 8 env warps
 
 // -DRF_TRACE (tools/rollout_trace.py builds that variant; never the shipped library): clock64 stamps of cluster 0's
 // first steps, one row per (CTA, step), read back through sb200_debug_rf_trace().
@@ -91,8 +97,6 @@ struct RfParams {
     // shared-memory plan (float offsets)
     int oW1, oW2, oWh, oB, oX0, oH1, oH2, oPart, oZf, oEnv, oS, oNext, oAct, oPre;
     int ldx0, ldh1, ldh2;
-    int l1_direct;                  // v2: reduction-free first layer (rf2_layer1)
-    int head_mode;                  // v2: 1 = k-sliced head over all owned actors, 0 = two warps per actor
 };
 
 __device__ __forceinline__ float rf_act(float v, int act) {
@@ -107,433 +111,12 @@ __device__ __forceinline__ unsigned rf_mapa(unsigned addr, unsigned rank) {
     asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
     return r;
 }
-__device__ __forceinline__ void rf_st_cluster_v4(unsigned addr, const float4& v) {
-    asm volatile("st.shared::cluster.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w)
-                 : "memory");
-}
-
-// One hidden layer for the cluster's 32 rows, this CTA's Nc columns: out[row][col0 + c] = act(x[row] . Ws[:, c] + b).
-// Xin [32][ldin] and Ws [K][Nc] live in shared memory; K % 4 == 0.
-//   Thread tile 4 rows x 4 columns (16 accumulators): with the first version's 1 x 4 tile every 16 FFMA needed 5
-//   LDS.128 and the layer was bound by shared-memory bandwidth (ncu: mio_throttle + short_scoreboard, 60 % of the
-//   kernel); 4 x 4 needs 8 LDS.128 per 64 FFMA.  The 512 threads form 4 groups of 128 that split K; the partial
-//   tiles are summed in a fixed order (deterministic) through `Part` [4][32][Nc].
-//   ALL_ROWS: the result is stored in every CTA's copy of Hout [32][ldout] (input of the next hidden layer);
-//   otherwise each row goes only to the CTA that owns the actor, into its Hout [8][ldout] (input of the head).
-template <bool ALL_ROWS, bool F2>
-__device__ __forceinline__ void rf_layer(const float* __restrict__ Xin, int ldin, int K, const float* __restrict__ Ws,
-                                         int Nc, const float* __restrict__ bias_s, int act, float* __restrict__ Hout,
-                                         int ldout, int col0, float* __restrict__ Part, unsigned smem_base,
-                                         unsigned crank, int rf_t, int rf_id) {
-    const int tid = threadIdx.x;
-    const int q = tid >> 7, t128 = tid & 127, ty = t128 >> 4, tx = t128 & 15;
-    const int kq = (((K >> 2) + 3) >> 2) << 2;               // k span of one group (multiple of 4)
-    const int k_lo = q * kq, k_hi = min(K, k_lo + kq);
-    const int nq = Nc >> 2;
-    for (int c4 = tx; c4 < nq; c4 += 16) {
-        const float* xr = Xin + (ty * 4) * ldin;
-        const float* wp = Ws + c4 * 4;
-        if constexpr (F2) {
-            // packed fma.rn.f32x2 (sm_100): two columns per instruction; each half is an IEEE fma, so the result is
-            // bit-identical to the scalar path -- it only halves the FFMA issue slots
-            float2 acc[4][2];
-#pragma unroll
-            for (int r = 0; r < 4; ++r) acc[r][0] = acc[r][1] = make_float2(0.0f, 0.0f);
-#pragma unroll 2
-            for (int k = k_lo; k < k_hi; k += 4) {
-                float4 a[4];
-#pragma unroll
-                for (int r = 0; r < 4; ++r) a[r] = *reinterpret_cast<const float4*>(xr + r * ldin + k);
-                const float4 w0 = *reinterpret_cast<const float4*>(wp + (k + 0) * Nc);
-                const float4 w1 = *reinterpret_cast<const float4*>(wp + (k + 1) * Nc);
-                const float4 w2 = *reinterpret_cast<const float4*>(wp + (k + 2) * Nc);
-                const float4 w3 = *reinterpret_cast<const float4*>(wp + (k + 3) * Nc);
-#pragma unroll
-                for (int r = 0; r < 4; ++r) {
-                    float2 aa = make_float2(a[r].x, a[r].x);
-                    acc[r][0] = __ffma2_rn(aa, make_float2(w0.x, w0.y), acc[r][0]);
-                    acc[r][1] = __ffma2_rn(aa, make_float2(w0.z, w0.w), acc[r][1]);
-                    aa = make_float2(a[r].y, a[r].y);
-                    acc[r][0] = __ffma2_rn(aa, make_float2(w1.x, w1.y), acc[r][0]);
-                    acc[r][1] = __ffma2_rn(aa, make_float2(w1.z, w1.w), acc[r][1]);
-                    aa = make_float2(a[r].z, a[r].z);
-                    acc[r][0] = __ffma2_rn(aa, make_float2(w2.x, w2.y), acc[r][0]);
-                    acc[r][1] = __ffma2_rn(aa, make_float2(w2.z, w2.w), acc[r][1]);
-                    aa = make_float2(a[r].w, a[r].w);
-                    acc[r][0] = __ffma2_rn(aa, make_float2(w3.x, w3.y), acc[r][0]);
-                    acc[r][1] = __ffma2_rn(aa, make_float2(w3.z, w3.w), acc[r][1]);
-                }
-            }
-#pragma unroll
-            for (int r = 0; r < 4; ++r)
-                *reinterpret_cast<float4*>(Part + ((q * RF_ROWS + ty * 4 + r) * Nc + c4 * 4)) =
-                    make_float4(acc[r][0].x, acc[r][0].y, acc[r][1].x, acc[r][1].y);
-        } else {
-        float acc[4][4];
-#pragma unroll
-        for (int r = 0; r < 4; ++r)
-#pragma unroll
-            for (int c = 0; c < 4; ++c) acc[r][c] = 0.0f;
-#pragma unroll 2
-        for (int k = k_lo; k < k_hi; k += 4) {
-            float4 a[4];
-#pragma unroll
-            for (int r = 0; r < 4; ++r) a[r] = *reinterpret_cast<const float4*>(xr + r * ldin + k);
-            const float4 w0 = *reinterpret_cast<const float4*>(wp + (k + 0) * Nc);
-            const float4 w1 = *reinterpret_cast<const float4*>(wp + (k + 1) * Nc);
-            const float4 w2 = *reinterpret_cast<const float4*>(wp + (k + 2) * Nc);
-            const float4 w3 = *reinterpret_cast<const float4*>(wp + (k + 3) * Nc);
-#pragma unroll
-            for (int r = 0; r < 4; ++r) {
-                acc[r][0] = fmaf(a[r].x, w0.x, acc[r][0]); acc[r][1] = fmaf(a[r].x, w0.y, acc[r][1]);
-                acc[r][2] = fmaf(a[r].x, w0.z, acc[r][2]); acc[r][3] = fmaf(a[r].x, w0.w, acc[r][3]);
-                acc[r][0] = fmaf(a[r].y, w1.x, acc[r][0]); acc[r][1] = fmaf(a[r].y, w1.y, acc[r][1]);
-                acc[r][2] = fmaf(a[r].y, w1.z, acc[r][2]); acc[r][3] = fmaf(a[r].y, w1.w, acc[r][3]);
-                acc[r][0] = fmaf(a[r].z, w2.x, acc[r][0]); acc[r][1] = fmaf(a[r].z, w2.y, acc[r][1]);
-                acc[r][2] = fmaf(a[r].z, w2.z, acc[r][2]); acc[r][3] = fmaf(a[r].z, w2.w, acc[r][3]);
-                acc[r][0] = fmaf(a[r].w, w3.x, acc[r][0]); acc[r][1] = fmaf(a[r].w, w3.y, acc[r][1]);
-                acc[r][2] = fmaf(a[r].w, w3.z, acc[r][2]); acc[r][3] = fmaf(a[r].w, w3.w, acc[r][3]);
-            }
-        }
-#pragma unroll
-        for (int r = 0; r < 4; ++r)
-            *reinterpret_cast<float4*>(Part + ((q * RF_ROWS + ty * 4 + r) * Nc + c4 * 4)) =
-                make_float4(acc[r][0], acc[r][1], acc[r][2], acc[r][3]);
-        }
-    }
-    RF_STAMP(rf_id, 0);
-    __syncthreads();
-    RF_STAMP(rf_id + 1, 0);
-    for (int idx = tid; idx < RF_ROWS * nq; idx += RF_THREADS) {
-        const int row = idx / nq, c4 = idx - row * nq;
-        const float* pp = Part + row * Nc + c4 * 4;
-        const float4 p0 = *reinterpret_cast<const float4*>(pp);
-        const float4 p1 = *reinterpret_cast<const float4*>(pp + RF_ROWS * Nc);
-        const float4 p2 = *reinterpret_cast<const float4*>(pp + 2 * RF_ROWS * Nc);
-        const float4 p3 = *reinterpret_cast<const float4*>(pp + 3 * RF_ROWS * Nc);
-        const float4 bv = *reinterpret_cast<const float4*>(bias_s + c4 * 4);
-        float4 o;
-        o.x = rf_act(((p0.x + p1.x) + (p2.x + p3.x)) + bv.x, act);
-        o.y = rf_act(((p0.y + p1.y) + (p2.y + p3.y)) + bv.y, act);
-        o.z = rf_act(((p0.z + p1.z) + (p2.z + p3.z)) + bv.z, act);
-        o.w = rf_act(((p0.w + p1.w) + (p2.w + p3.w)) + bv.w, act);
-        if (ALL_ROWS) {
-            float* qd = Hout + row * ldout + col0 + c4 * 4;
-            *reinterpret_cast<float4*>(qd) = o;
-            const unsigned off = rf_smem_u32(qd) - smem_base;
-#pragma unroll
-            for (int c = 1; c < RF_CS; ++c) rf_st_cluster_v4(rf_mapa(smem_base, (crank + (unsigned)c) % RF_CS) + off, o);
-        } else {
-            const unsigned owner = (unsigned)(row / RF_OWN);
-            float* qd = Hout + (row - (int)owner * RF_OWN) * ldout + col0 + c4 * 4;
-            if (owner == crank) *reinterpret_cast<float4*>(qd) = o;
-            else rf_st_cluster_v4(rf_mapa(smem_base, owner) + (rf_smem_u32(qd) - smem_base), o);
-        }
-    }
-}
-
-template <bool F2>
-__global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
-    ppo_rollout_kernel(const __grid_constant__ RfParams p) {
-    cg::cluster_group cluster = cg::this_cluster();
-    const unsigned crank = cluster.block_rank();
-    extern __shared__ __align__(16) float smem[];
-    const unsigned smem_base = rf_smem_u32(smem);
-    unsigned peer_base[RF_CS - 1];
-#pragma unroll
-    for (int c = 1; c < RF_CS; ++c) peer_base[c - 1] = rf_mapa(smem_base, (crank + (unsigned)c) % RF_CS);
-    __shared__ int s_pos[RF_OWN], s_ep[RF_OWN], s_cnt[RF_OWN];
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int D = p.D, H1 = p.H1, H2 = p.H2, A = p.A;
-    const int Nc1 = H1 / RF_CS, Nc2 = H2 / RF_CS;
-    const int ldwh = p.ldw[2];
-    float* W1s = smem + p.oW1;          // [D][Nc1]
-    float* W2s = smem + p.oW2;          // [H1][Nc2]
-    float* Whs = smem + p.oWh;          // [H2][ldwh]
-    float* B1s = smem + p.oB;           // [Nc1] | [Nc2] | [ldwh]
-    float* B2s = B1s + Nc1;
-    float* Bhs = B2s + Nc2;
-    float* X0 = smem + p.oX0;           // [32][ldx0]  z-filtered observations of the cluster's actors
-    float* Hb1 = smem + p.oH1;          // [32][ldh1]
-    float* Hb2 = smem + p.oH2;          // [8][ldh2]   last hidden layer, owned actors only
-    float* Part = smem + p.oPart;       // [4][32][max(Nc1, Nc2)] k-split partial tiles
-    float* Zm = smem + p.oZf;           // [D] mean | [D] std
-    float* Zs = Zm + D;
-    float* EWs = smem + p.oEnv;         // [D][D] | [A][D]   (k-major)
-    float* EWa = EWs + D * D;
-    float* S = smem + p.oS;             // [8][D]   env state of the owned actors (what they observe next)
-    float* Nx = smem + p.oNext;         // [8][D]   true successor of the step
-    float* Ac = smem + p.oAct;          // [8][A]   sampled actions | means | std | N(0,1) draws
-    float* Mu = Ac + RF_OWN * A;
-    float* Sd = Mu + RF_OWN * A;
-    float* Zn = Sd + RF_OWN * A;
-    float* Eacc = smem + p.oPre;        // [8][D] Ws.s | [8][D] env noise | [8][D] reset draws | [16] |s|^2, reward noise
-    float* Egx = Eacc + RF_OWN * D;
-    float* Erz = Egx + RF_OWN * D;
-    float* Eq = Erz + RF_OWN * D;
-    const long long row0 = (long long)(blockIdx.x / RF_CS) * RF_ROWS;
-
-    // ---- one-time loads: weight slices, biases, env matrices (cp.async burst), z-filter columns, actor state
-    for (int f = tid; f < D * (Nc1 >> 2); f += RF_THREADS) {
-        const int k = f / (Nc1 >> 2), q = f - k * (Nc1 >> 2);
-        cp_async16(W1s + k * Nc1 + q * 4, p.W[0] + (long long)k * p.ldw[0] + crank * Nc1 + q * 4, 16);
-    }
-    for (int f = tid; f < H1 * (Nc2 >> 2); f += RF_THREADS) {
-        const int k = f / (Nc2 >> 2), q = f - k * (Nc2 >> 2);
-        cp_async16(W2s + k * Nc2 + q * 4, p.W[1] + (long long)k * p.ldw[1] + crank * Nc2 + q * 4, 16);
-    }
-    for (int f = tid; f < (H2 * ldwh) >> 2; f += RF_THREADS) cp_async16(Whs + f * 4, p.W[2] + f * 4, 16);
-    for (int f = tid; f < (D * D) >> 2; f += RF_THREADS) cp_async16(EWs + f * 4, p.WsT + f * 4, 16);
-    for (int f = tid; f < (A * D) >> 2; f += RF_THREADS) cp_async16(EWa + f * 4, p.WaT + f * 4, 16);
-    cp_async_commit();
-    for (int n = tid; n < Nc1; n += RF_THREADS) B1s[n] = p.b[0][crank * Nc1 + n];
-    for (int n = tid; n < Nc2; n += RF_THREADS) B2s[n] = p.b[1][crank * Nc2 + n];
-    for (int n = tid; n < ldwh; n += RF_THREADS) Bhs[n] = (n < A) ? p.b[2][n] : 0.0f;
-    if (p.zf != nullptr) {
-        const float cnt = p.zf[2 * D];
-        for (int k = tid; k < D; k += RF_THREADS) {
-            const float mean = p.zf[k] / cnt;
-            const float var = p.zf[D + k] / cnt - mean * mean;
-            Zm[k] = mean;
-            Zs[k] = fmaxf(sqrtf(var), p.zf_eps);
-        }
-    }
-    if (tid < RF_OWN) {
-        const long long i = row0 + crank * RF_OWN + tid;
-        s_pos[tid] = (i < p.N) ? p.stage_pos[i] : 0;
-        s_ep[tid] = (i < p.N) ? p.ep_step[i] : 0;
-        s_cnt[tid] = 0;
-    }
-    __syncthreads();
-    for (int idx = tid; idx < RF_ROWS * D; idx += RF_THREADS) {       // all 32 rows: every CTA needs the full input
-        const int m = idx / D, k = idx - m * D;
-        const long long i = row0 + m;
-        float v = (i < p.N) ? p.state[i * D + k] : 0.0f;
-        const int own = m - (int)crank * RF_OWN;
-        if (own >= 0 && own < RF_OWN) S[own * D + k] = v;
-        if (p.zf != nullptr) v = fminf(fmaxf((v - Zm[k]) / Zs[k], -5.0f), 5.0f);
-        X0[m * p.ldx0 + k] = (i < p.N) ? v : 0.0f;
-    }
-    const unsigned long long ctr0 = (p.step_ctr != nullptr) ? *p.step_ctr : 0ull;
-    cp_async_wait<0>();
-    cluster.sync();                                   // weights landed; every peer is running (DSMEM is live)
-
-    const int own = warp;                             // warps 0..7: one owned actor each
-    const bool owner = own < RF_OWN;
-    const int m_own = (int)crank * RF_OWN + own;
-    const long long i_own = row0 + m_own;
-    const bool valid = owner && (i_own < p.N);
-    const float sc = (valid && p.log_noise != nullptr) ? expf(p.log_noise[i_own]) : 1.0f;
-    if (owner && lane < A) Sd[own * A + lane] = __fmul_rn(expf(p.log_var[lane]), sc);     // constant over the chunk
-    __syncthreads();
-
-    for (int t = 0; t < p.T; ++t) {
-        const unsigned long long ctr = ctr0 + (unsigned long long)t;
-        const bool final_step = (t == p.T - 1);
-        const int rf_t = t;
-        RF_STAMP(0, 0);
-        rf_layer<true, F2>(X0, p.ldx0, D, W1s, Nc1, B1s, p.act[0], Hb1, p.ldh1, (int)crank * Nc1, Part, smem_base, crank, rf_t, 1);
-        RF_STAMP(3, 0);
-        cluster.sync();
-        RF_STAMP(4, 0);
-        rf_layer<false, F2>(Hb1, p.ldh1, H1, W2s, Nc2, B2s, p.act[1], Hb2, p.ldh2, (int)crank * Nc2, Part, smem_base, crank, rf_t, 5);
-        RF_STAMP(7, 0);
-        cluster.sync();
-        RF_STAMP(8, 0);
-        RF_STAMP(16, 256);
-
-        float rew = 0.0f, dn = 0.0f;
-        int slot = SLOT_NONE;
-        // ---- phase 1, two halves of the CTA in parallel.  Owner warps 0..7: the head.  Helper warps 8..15 (one per
-        // owned actor): everything of the step that does not depend on the action -- the exploration draws, Ws.s, the
-        // env noise, |s|^2 -- so that the serial chain after the head is a handful of instructions.
-        if (owner) {
-            const float* hrow = Hb2 + own * p.ldh2;
-            for (int n8 = 0; n8 < A; n8 += 8) {
-                float s8[8];
-#pragma unroll
-                for (int jj = 0; jj < 8; ++jj) s8[jj] = 0.0f;
-                const bool second = (n8 + 4 < ldwh);
-                for (int k = lane; k < H2; k += 32) {
-                    const float hv = hrow[k];
-                    const float* wr = Whs + k * ldwh + n8;
-                    const float4 w0 = *reinterpret_cast<const float4*>(wr);
-                    s8[0] = fmaf(hv, w0.x, s8[0]); s8[1] = fmaf(hv, w0.y, s8[1]);
-                    s8[2] = fmaf(hv, w0.z, s8[2]); s8[3] = fmaf(hv, w0.w, s8[3]);
-                    if (second) {
-                        const float4 w1 = *reinterpret_cast<const float4*>(wr + 4);
-                        s8[4] = fmaf(hv, w1.x, s8[4]); s8[5] = fmaf(hv, w1.y, s8[5]);
-                        s8[6] = fmaf(hv, w1.z, s8[6]); s8[7] = fmaf(hv, w1.w, s8[7]);
-                    }
-                }
-                float mine = 0.0f;
-#pragma unroll
-                for (int jj = 0; jj < 8; ++jj) {
-                    const float tt = warp_sum(s8[jj]);
-                    if (lane == jj) mine = tt;
-                }
-                const int j = n8 + lane;
-                if (lane < 8 && j < A) Mu[own * A + j] = rf_act(mine + Bhs[j], p.act[2]);
-            }
-        } else {
-            const int h = warp - RF_OWN;                       // helper of owned actor h
-            const long long ih = row0 + (int)crank * RF_OWN + h;
-            const float* sh = S + h * D;
-            float q = 0.0f;
-            for (int d = lane; d < D; d += 32) q += sh[d] * sh[d];
-            q = warp_sum(q);
-            const bool h_done = (p.max_steps > 0) && (s_ep[h] + 1 >= p.max_steps);
-            for (int d = lane; d < D; d += 32) {
-                float acc = 0.0f;                              // WsT is [k][d]: conflict-free across lanes
-#pragma unroll 8
-                for (int k = 0; k < D; ++k) acc = fmaf(EWs[k * D + d], sh[k], acc);
-                const Philox4 r = philox4x32_10(p.env_seed ^ 0x5851F42D4C957F2Dull, ctr,
-                                                ((unsigned long long)ih << 20) | (unsigned long long)d);
-                const float2 gz = box_muller(r.x, r.y);
-                Eacc[h * D + d] = acc;
-                Egx[h * D + d] = gz.x;
-                Erz[h * D + d] = h_done ? box_muller(r.z, r.w).x : 0.0f;
-                if (d == 0) {
-                    Eq[2 * h] = q;
-                    Eq[2 * h + 1] = gz.y;
-                }
-            }
-            if (!p.deterministic && lane < A) {                // PPOAgent.act's N(0,1) draws: keys of sample_one()
-                const int j = lane;
-                const Philox4 r = philox4x32_10(p.agent_seed, ctr, ((unsigned long long)ih << 16) | (unsigned long long)(j >> 2));
-                const float2 z01 = box_muller(r.x, r.y), z23 = box_muller(r.z, r.w);
-                const int c = j & 3;
-                Zn[h * A + j] = (c == 0) ? z01.x : (c == 1) ? z01.y : (c == 2) ? z23.x : z23.y;
-            }
-        }
-        RF_STAMP(9, 0);
-        RF_STAMP(17, 256);
-        __syncthreads();
-        RF_STAMP(10, 0);
-        // ---- phase 2 (owner warps): action, env step, bookkeeping -- same arithmetic, operand order and Philox keys as
-        // sample_one() / synth_env_block() of rollout.cu
-        if (owner) {
-            const int pos = s_pos[own];
-            if (lane < A) {
-                const int j = lane;
-                const float mu = Mu[own * A + j];
-                const float sd = Sd[own * A + j];
-                float a = mu;
-                if (!p.deterministic) a = __fadd_rn(__fmul_rn(Zn[own * A + j], sd), mu);
-                a = fminf(fmaxf(a, -1.0f), 1.0f);
-                Ac[own * A + j] = a;
-                if (valid) {
-                    p.stage_act[((long long)i_own * p.n_step + pos) * A + j] = a;
-                    p.stage_pd[((long long)i_own * p.n_step + pos) * 2 * A + j] = mu;
-                    p.stage_pd[((long long)i_own * p.n_step + pos) * 2 * A + A + j] = sd;
-                    if (final_step) {
-                        p.action[i_own * A + j] = a;
-                        p.pd[i_own * 2 * A + j] = mu;
-                        p.pd[i_own * 2 * A + A + j] = sd;
-                    }
-                }
-            }
-            __syncwarp();
-            float* sown = S + own * D;
-            const int ep = s_ep[own] + 1;
-            const bool is_done = (p.max_steps > 0) && (ep >= p.max_steps);
-            dn = is_done ? 1.0f : 0.0f;
-            rew = -Eq[2 * own] / (float)D + 0.1f * Eq[2 * own + 1];
-            for (int d = lane; d < D; d += 32) {
-                float acc = Eacc[own * D + d];
-#pragma unroll 4
-                for (int k = 0; k < A; ++k) acc = fmaf(EWa[k * D + d], Ac[own * A + k], acc);
-                const float nxt = tanhf(acc) + 0.01f * Egx[own * D + d];
-                Nx[own * D + d] = nxt;
-                sown[d] = is_done ? Erz[own * D + d] : nxt;
-                if (valid && final_step) p.obs_next[i_own * D + d] = nxt;
-            }
-            if (lane == 0) {
-                s_ep[own] = is_done ? 0 : ep;
-                if (valid && final_step) {
-                    p.reward[i_own] = rew;
-                    p.done[i_own] = dn;
-                }
-                if (valid && pos + 1 == p.n_step) {            // this step completes a window -> next outbox entry
-                    const int w = s_cnt[own];
-                    if (w < p.Wout) {
-                        slot = (int)(i_own * p.Wout + w);
-                        p.ev_step[slot] = t;
-                        s_cnt[own] = w + 1;
-                    } else {
-                        slot = SLOT_DROPPED;
-                    }
-                }
-            }
-            slot = __shfl_sync(0xffffffffu, slot, 0);
-            __syncwarp();
-        }
-        RF_STAMP(11, 0);
-        // ---- window staging (block-wide barriers inside: every warp calls; only owners do work)
-        commit_actor(valid, (int)i_own, lane, 32, Nx + (owner ? own : 0) * D, S + (owner ? own : 0) * D, rew, dn, p.n_step,
-                     p.stride, D, A, s_pos + (owner ? own : 0), slot, p.stage_obs, p.stage_act, p.stage_pd, p.stage_rew,
-                     p.stage_done, p.o_obs, p.o_act, p.o_pd, p.o_rew, p.o_done);
-        RF_STAMP(12, 0);
-        // ---- next observation -> z-filter -> every CTA's input tile
-        if (owner) {
-            const int q4 = lane;                            // D / 4 <= 32 float4 per row
-            if (q4 < (D >> 2)) {
-                float4 v = *reinterpret_cast<const float4*>(S + own * D + q4 * 4);
-                if (i_own >= p.N) v = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (p.zf != nullptr) {
-                    const float4 zm = *reinterpret_cast<const float4*>(Zm + q4 * 4);
-                    const float4 zs = *reinterpret_cast<const float4*>(Zs + q4 * 4);
-                    v.x = fminf(fmaxf((v.x - zm.x) / zs.x, -5.0f), 5.0f);
-                    v.y = fminf(fmaxf((v.y - zm.y) / zs.y, -5.0f), 5.0f);
-                    v.z = fminf(fmaxf((v.z - zm.z) / zs.z, -5.0f), 5.0f);
-                    v.w = fminf(fmaxf((v.w - zm.w) / zs.w, -5.0f), 5.0f);
-                    if (i_own >= p.N) v = make_float4(0.f, 0.f, 0.f, 0.f);
-                }
-                float* qx = X0 + m_own * p.ldx0 + q4 * 4;
-                *reinterpret_cast<float4*>(qx) = v;
-                const unsigned off = rf_smem_u32(qx) - smem_base;
-#pragma unroll
-                for (int c = 0; c < RF_CS - 1; ++c) rf_st_cluster_v4(peer_base[c] + off, v);
-            }
-        }
-        RF_STAMP(13, 0);
-        cluster.sync();
-        RF_STAMP(14, 0);
-    }
-
-    // ---- write the per-actor control state back
-    if (valid) {
-        for (int d = lane; d < D; d += 32) p.state[i_own * D + d] = S[own * D + d];
-        if (lane == 0) {
-            p.stage_pos[i_own] = s_pos[own];
-            p.ep_step[i_own] = s_ep[own];
-            p.ev_count[i_own] = s_cnt[own];
-        }
-    }
-}
-
-
-// =====================================================================================================================
-// v2 of the persistent rollout kernel: same cluster / resident-weight / DSMEM structure, same arithmetic for sampling and
-// the environment, two changes of schedule that the clock64 trace of v1 asked for (tools/rollout_trace.py):
-//   * WARP SPECIALISATION.  In v1 the action-independent half of the env step (Philox + Box-Muller draws, Ws.s, |s|^2:
-//     ~6.8 K cycles on 8 helper warps) sat on the serial chain behind the layers.  Now warps 0..7 ("math warps") run
-//     the two hidden layers while warps 8..15 ("env warps") do that work for the SAME step concurrently -- it depends
-//     only on the state at the top of the step.  The env warps arrive at cluster barrier 1 before they start
-//     (barrier.cluster.arrive / .wait are split-phase), so they never hold the math warps up.
-//   * 8 x 4 REGISTER TILES in the layers (was 4 x 4): 12 LDS.128 per 128 FMA instead of 8 per 64 -- the layer loop was
-//     bound by shared-memory loads, not by FFMA issue.  A warp = 16 column quads x 2 k-halves over ONE 8-row group, so
-//     the activation loads are warp-wide broadcasts.
-//   * the head runs on all 16 warps (2 per owned actor, k halves) with a 9-shuffle transposing reduction.
 __device__ __forceinline__ void rf_bar_math() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
-__device__ __forceinline__ void rf_cluster_arrive() { asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory"); }
-__device__ __forceinline__ void rf_cluster_wait() { asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory"); }
 
-// ---- mbarrier-signalled DSMEM hand-off (the ASYNC variant of the v2 kernel).  barrier.cluster.arrive.release compiles to
-// MEMBAR.ALL.GPU + ERRBAR + CGAERRBAR in front of the barrier (the kernel's global stores of the step must drain to L2
-// first) and the wait to a CCTL.IVALL: three times per env step.  st.async carries the data AND the completion count to
-// the consumer's mbarrier, so the producer needs no fence and the consumer polls its own shared memory.
+// ---- mbarrier-signalled DSMEM hand-off.  st.async carries the data AND the completion count to the consumer's
+// mbarrier, so the producer needs no fence and the consumer polls its own shared memory.  (barrier.cluster.arrive.release
+// would compile to MEMBAR.ALL.GPU + ERRBAR + CGAERRBAR in front of the barrier -- the kernel's global stores of the step
+// must drain to L2 first -- and the wait to a CCTL.IVALL: three times per env step.)
 __device__ __forceinline__ void rf_mbar_init(unsigned long long* bar, unsigned count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(rf_smem_u32(bar)), "r"(count) : "memory");
 }
@@ -560,33 +143,18 @@ __device__ __forceinline__ void rf_st_async_v4(unsigned dst_cluster_addr, const 
                  ::"r"(dst_cluster_addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w), "r"(mbar_cluster_addr) : "memory");
 }
 
-// sum over the 32 lanes of s[j], returned in the lanes with j == 4*bit4 + 2*bit3 + bit2 of the lane index (9 shuffles)
-__device__ __forceinline__ float rf_reduce8(const float (&s)[8], int lane) {
-    const bool u4 = (lane & 16) != 0, u3 = (lane & 8) != 0, u2 = (lane & 4) != 0;
-    float t[4], u[2];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const float recv = __shfl_xor_sync(0xffffffffu, u4 ? s[i] : s[i + 4], 16);
-        t[i] = (u4 ? s[i + 4] : s[i]) + recv;
-    }
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-        const float recv = __shfl_xor_sync(0xffffffffu, u3 ? t[i] : t[i + 2], 8);
-        u[i] = (u3 ? t[i + 2] : t[i]) + recv;
-    }
-    float v = (u2 ? u[1] : u[0]) + __shfl_xor_sync(0xffffffffu, u2 ? u[0] : u[1], 4);
-    v += __shfl_xor_sync(0xffffffffu, v, 2);
-    v += __shfl_xor_sync(0xffffffffu, v, 1);
-    return v;
-}
-
-// One hidden layer on the 8 math warps (tid 0..255): warp = (row group rg = warp & 3: rows 8rg..8rg+7, k quarter pair),
-// lane = (column quad, k half) -> 4-way k split, partial tiles summed in a fixed order through Part [4][32][Nc].
-template <bool ALL_ROWS, bool ASYNC>
+// The last hidden layer on the 8 math warps (tid 0..255), this CTA's Nc columns for the cluster's 32 rows; each row goes
+// only to the CTA that owns the actor, into its Hout [8][ldout] (input of the head).  Xin [32][ldin] and Ws [K][Nc] live
+// in shared memory; K % 4 == 0.
+//   warp = (row group rg = warp & 3: rows 8rg..8rg+7, k quarter pair), lane = (column quad, k half) -> 4-way k split,
+//   partial tiles summed in a fixed order (deterministic) through Part [4][32][Nc].  8 x 4 register tiles: 12 LDS.128 per
+//   128 FMA -- the layer loop is bound by shared-memory loads, not by FMA issue -- and the activation loads of a warp
+//   (ONE 8-row group) are warp-wide broadcasts.  Packed fma.rn.f32x2: each half is an IEEE fma, so the result is that
+//   of two scalar fmaf; it only halves the issue slots.
 __device__ __forceinline__ void rf2_layer(const float* __restrict__ Xin, int ldin, int K, const float* __restrict__ Ws,
                                           int Nc, const float* __restrict__ bias_s, int act, float* __restrict__ Hout,
                                           int ldout, int col0, float* __restrict__ Part, unsigned smem_base,
-                                          unsigned crank, int rf_t, int rf_id, unsigned bar_off) {
+                                          unsigned crank, int rf_t, unsigned bar_off) {
     const int tid = (int)RF_TID, warp = tid >> 5, lane = tid & 31;
     const int rg = warp & 3, ks = ((warp >> 2) << 1) | (lane >> 4), cg0 = lane & 15;
     const int kq = (((K >> 2) + 3) >> 2) << 2;               // k span of one split (multiple of 4)
@@ -626,9 +194,9 @@ __device__ __forceinline__ void rf2_layer(const float* __restrict__ Xin, int ldi
             *reinterpret_cast<float4*>(Part + ((ks * RF_ROWS + rg * 8 + r) * Nc + c4 * 4)) =
                 make_float4(acc[r][0].x, acc[r][0].y, acc[r][1].x, acc[r][1].y);
     }
-    RF_STAMP(rf_id, 0);
+    RF_STAMP(5, 0);
     rf_bar_math();
-    RF_STAMP(rf_id + 1, 0);
+    RF_STAMP(6, 0);
     for (int idx = tid; idx < RF_ROWS * nq; idx += 256) {
         const int row = idx / nq, c4 = idx - row * nq;
         const float* pp = Part + row * Nc + c4 * 4;
@@ -642,38 +210,25 @@ __device__ __forceinline__ void rf2_layer(const float* __restrict__ Xin, int ldi
         o.y = rf_act(((p0.y + p1.y) + (p2.y + p3.y)) + bv.y, act);
         o.z = rf_act(((p0.z + p1.z) + (p2.z + p3.z)) + bv.z, act);
         o.w = rf_act(((p0.w + p1.w) + (p2.w + p3.w)) + bv.w, act);
-        if (ALL_ROWS) {
-            float* qd = Hout + row * ldout + col0 + c4 * 4;
+        const unsigned owner = (unsigned)(row / RF_OWN);
+        float* qd = Hout + (row - (int)owner * RF_OWN) * ldout + col0 + c4 * 4;
+        if (owner == crank) {
             *reinterpret_cast<float4*>(qd) = o;
-            const unsigned off = rf_smem_u32(qd) - smem_base;
-#pragma unroll
-            for (int c = 1; c < RF_CS; ++c) {
-                const unsigned pb = rf_mapa(smem_base, (crank + (unsigned)c) % RF_CS);
-                if (ASYNC) rf_st_async_v4(pb + off, o, pb + bar_off);
-                else rf_st_cluster_v4(pb + off, o);
-            }
         } else {
-            const unsigned owner = (unsigned)(row / RF_OWN);
-            float* qd = Hout + (row - (int)owner * RF_OWN) * ldout + col0 + c4 * 4;
-            if (owner == crank) {
-                *reinterpret_cast<float4*>(qd) = o;
-            } else {
-                const unsigned pb = rf_mapa(smem_base, owner);
-                if (ASYNC) rf_st_async_v4(pb + (rf_smem_u32(qd) - smem_base), o, pb + bar_off);
-                else rf_st_cluster_v4(pb + (rf_smem_u32(qd) - smem_base), o);
-            }
+            const unsigned pb = rf_mapa(smem_base, owner);
+            rf_st_async_v4(pb + (rf_smem_u32(qd) - smem_base), o, pb + bar_off);
         }
     }
 }
 
 // First hidden layer on the 8 math warps WITHOUT a shared-memory reduction: K = D is short (64), so the 4-way k split of
-// rf2_layer spent more on partial tiles, the barrier and the second pass (1.5 K cycles) than on its 4 k quads of FMAs.
-// Here warp w owns rows 4w..4w+3, lane = (column quad, k half); the two k halves of a lane pair are summed by shuffle
-// (each lane keeps two of the four rows) and the epilogue stores / pushes straight from registers.
-template <bool ASYNC>
+// rf2_layer would spend more on partial tiles, the barrier and the second pass (1.5 K cycles) than on its 4 k quads of
+// FMAs.  Warp w owns rows 4w..4w+3, lane = (column quad, k half); the two k halves of a lane pair are summed by shuffle
+// (each lane keeps two of the four rows) and the epilogue stores / pushes the result into every CTA's copy of
+// Hout [32][ldout] straight from registers.
 __device__ __forceinline__ void rf2_layer1(const float* __restrict__ Xin, int ldin, int K, const float* __restrict__ Ws, int Nc,
                                            const float* __restrict__ bias_s, int act, float* __restrict__ Hout, int ldout,
-                                           int col0, unsigned smem_base, unsigned crank, unsigned bar_off, int rf_t) {
+                                           int col0, unsigned smem_base, unsigned crank, unsigned bar_off) {
     const int tid = (int)RF_TID, warp = tid >> 5, lane = tid & 31;
     const int cg0 = lane & 15, kh = lane >> 4;
     const bool up = kh != 0;
@@ -729,18 +284,12 @@ __device__ __forceinline__ void rf2_layer1(const float* __restrict__ Xin, int ld
                 *reinterpret_cast<float4*>(qd) = o;
                 const unsigned off = rf_smem_u32(qd) - smem_base;
 #pragma unroll
-                for (int c = 0; c < RF_CS - 1; ++c) {
-                    if (ASYNC) rf_st_async_v4(pb[c] + off, o, pb[c] + bar_off);
-                    else rf_st_cluster_v4(pb[c] + off, o);
-                }
+                for (int c = 0; c < RF_CS - 1; ++c) rf_st_async_v4(pb[c] + off, o, pb[c] + bar_off);
             }
         }
     }
-    RF_STAMP(1, 0);
-    RF_STAMP(2, 0);
 }
 
-template <bool ASYNC>
 __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
     ppo_rollout2_kernel(const __grid_constant__ RfParams p) {
     cg::cluster_group cluster = cg::this_cluster();
@@ -751,7 +300,7 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
 #pragma unroll
     for (int c = 1; c < RF_CS; ++c) peer_base[c - 1] = rf_mapa(smem_base, (crank + (unsigned)c) % RF_CS);
     __shared__ int s_pos[RF_OWN], s_ep[RF_OWN], s_cnt[RF_OWN];
-    __shared__ __align__(8) unsigned long long s_bar[3];      // ASYNC: hidden layer 1 | last hidden layer rows | next input tile
+    __shared__ __align__(8) unsigned long long s_bar[3];      // hidden layer 1 | last hidden layer rows | next input tile
 
     // (tried: the two roles on swapped warp halves, in case the scheduler's preference for one end of the warp index range
     // starved the layers -- no difference, profiles/r02b_rollout_trace_*)
@@ -759,33 +308,32 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
     const int D = p.D, H1 = p.H1, H2 = p.H2, A = p.A;
     const int Nc1 = H1 / RF_CS, Nc2 = H2 / RF_CS;
     const int ldwh = p.ldw[2];
-    float* W1s = smem + p.oW1;
-    float* W2s = smem + p.oW2;
-    float* Whs = smem + p.oWh;
-    float* B1s = smem + p.oB;
+    float* W1s = smem + p.oW1;          // [D][Nc1]
+    float* W2s = smem + p.oW2;          // [H1][Nc2]
+    float* Whs = smem + p.oWh;          // [H2][ldwh]
+    float* B1s = smem + p.oB;           // [Nc1] | [Nc2] | [ldwh]
     float* B2s = B1s + Nc1;
     float* Bhs = B2s + Nc2;
-    float* X0 = smem + p.oX0;
-    float* Hb1 = smem + p.oH1;
-    float* Hb2 = smem + p.oH2;
-    float* Part = smem + p.oPart;
-    float* Zm = smem + p.oZf;
+    float* X0 = smem + p.oX0;           // [32][ldx0]  z-filtered observations of the cluster's actors
+    float* Hb1 = smem + p.oH1;          // [32][ldh1]
+    float* Hb2 = smem + p.oH2;          // [8][ldh2]   last hidden layer, owned actors only
+    float* Part = smem + p.oPart;       // [4][32][max(Nc1, Nc2)] k-split partial tiles | [16][8][ldwh] head slice sums
+    float* Zm = smem + p.oZf;           // [D] mean | [D] std
     float* Zs = Zm + D;
-    float* EWs = smem + p.oEnv;
+    float* EWs = smem + p.oEnv;         // [D][D] | [A][D]   (k-major)
     float* EWa = EWs + D * D;
-    float* S = smem + p.oS;
-    float* Nx = smem + p.oNext;
-    float* Ac = smem + p.oAct;
-    float* Sd = Ac + 2 * RF_OWN * A;     // (slot 1 = Mu of v1: unused here)
+    float* S = smem + p.oS;             // [8][D]   env state of the owned actors (what they observe next)
+    float* Nx = smem + p.oNext;         // [8][D]   true successor of the step
+    float* Ac = smem + p.oAct;          // [8][A]   sampled actions | std | N(0,1) draws
+    float* Sd = Ac + RF_OWN * A;
     float* Zn = Sd + RF_OWN * A;
-    float* Hp = Zn + RF_OWN * A;         // [2][8][A] head partial sums of the two k halves
-    float* Eacc = smem + p.oPre;
+    float* Eacc = smem + p.oPre;        // [8][D] Ws.s | [8][D] env noise | [8][D] reset draws | [16] |s|^2, reward noise
     float* Egx = Eacc + RF_OWN * D;
     float* Erz = Egx + RF_OWN * D;
     float* Eq = Erz + RF_OWN * D;
     const long long row0 = (long long)(blockIdx.x / RF_CS) * RF_ROWS;
 
-    // ---- one-time loads (as v1)
+    // ---- one-time loads: weight slices, biases, env matrices (cp.async burst), z-filter columns, actor state
     for (int f = tid; f < D * (Nc1 >> 2); f += RF_THREADS) {
         const int k = f / (Nc1 >> 2), q = f - k * (Nc1 >> 2);
         cp_async16(W1s + k * Nc1 + q * 4, p.W[0] + (long long)k * p.ldw[0] + crank * Nc1 + q * 4, 16);
@@ -817,7 +365,7 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
         s_cnt[tid] = 0;
     }
     __syncthreads();
-    for (int idx = tid; idx < RF_ROWS * D; idx += RF_THREADS) {
+    for (int idx = tid; idx < RF_ROWS * D; idx += RF_THREADS) {       // all 32 rows: every CTA needs the full input
         const int m = idx / D, k = idx - m * D;
         const long long i = row0 + m;
         float v = (i < p.N) ? p.state[i * D + k] : 0.0f;
@@ -827,17 +375,18 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
         X0[m * p.ldx0 + k] = (i < p.N) ? v : 0.0f;
     }
     const unsigned long long ctr0 = (p.step_ctr != nullptr) ? *p.step_ctr : 0ull;
-    if (ASYNC && tid == 0) {
+    if (tid == 0) {
         for (int i = 0; i < 3; ++i) rf_mbar_init(&s_bar[i], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     const unsigned bar_off_h1 = rf_smem_u32(&s_bar[0]) - smem_base, bar_off_h2 = rf_smem_u32(&s_bar[1]) - smem_base;
     const unsigned bar_off_x0 = rf_smem_u32(&s_bar[2]) - smem_base;
     // bytes a CTA receives from its three peers per step: their column quarters of hidden layer 1 for all 32 rows, their
-    // column quarters of the last hidden layer for the 8 owned rows, their 8 rows of the next input tile
+    // column quarters of the last hidden layer for the 8 owned rows, their 8 rows of the next input tile (each below the
+    // mbarrier's 2^20 transaction limit: rf_plan)
     const unsigned tx_h1 = 3u * RF_ROWS * Nc1 * 4u, tx_h2 = 3u * RF_OWN * Nc2 * 4u, tx_x0 = 3u * RF_OWN * D * 4u;
     cp_async_wait<0>();
-    cluster.sync();
+    cluster.sync();                                   // weights landed; barriers initialised; every peer is running
 
     const bool math = warp < RF_OWN;                  // warps 0..7: layers, then owner of actor `warp`
     const int own = warp & (RF_OWN - 1);              // owned actor this warp works for (owner or env warp)
@@ -847,7 +396,7 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
     const bool valid = owner && (i_own < p.N);
     {
         const float sc = (i_own < p.N && p.log_noise != nullptr) ? expf(p.log_noise[i_own]) : 1.0f;
-        if (owner && lane < A) Sd[own * A + lane] = __fmul_rn(expf(p.log_var[lane]), sc);
+        if (owner && lane < A) Sd[own * A + lane] = __fmul_rn(expf(p.log_var[lane]), sc);     // constant over the chunk
     }
     __syncthreads();
 
@@ -856,43 +405,28 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
         const bool final_step = (t == p.T - 1);
         const int rf_t = t;
         RF_STAMP(0, 0);
-        if (ASYNC && tid == 0) {                              // arm this step's phases (the previous ones were consumed)
+        if (tid == 0) {                                       // arm this step's phases (the previous ones were consumed)
             rf_mbar_arm(&s_bar[0], tx_h1);
             rf_mbar_arm(&s_bar[1], tx_h2);
         }
         if (math) {
-            if (ASYNC && t > 0) {                             // the input tile: own rows (math warps wrote them) + the peers' rows
+            if (t > 0) {                                      // the input tile: own rows (math warps wrote them) + the peers' rows
                 rf_bar_math();
                 rf_mbar_wait(&s_bar[2], (unsigned)(t - 1) & 1u);
             }
             RF_STAMP(18, 0);
-            if (ASYNC && tid == 0 && !final_step) rf_mbar_arm(&s_bar[2], tx_x0);     // next tile's phase: only now is the previous one complete
-            if (p.l1_direct)                                   // 8 math warps x 4 rows: the reduction-free form
-                rf2_layer1<ASYNC>(X0, p.ldx0, D, W1s, Nc1, B1s, p.act[0], Hb1, p.ldh1, (int)crank * Nc1, smem_base, crank, bar_off_h1, rf_t);
-            else
-                rf2_layer<true, ASYNC>(X0, p.ldx0, D, W1s, Nc1, B1s, p.act[0], Hb1, p.ldh1, (int)crank * Nc1, Part, smem_base, crank, rf_t, 1,
-                                       bar_off_h1);
+            if (tid == 0 && !final_step) rf_mbar_arm(&s_bar[2], tx_x0);     // next tile's phase: only now is the previous one complete
+            rf2_layer1(X0, p.ldx0, D, W1s, Nc1, B1s, p.act[0], Hb1, p.ldh1, (int)crank * Nc1, smem_base, crank, bar_off_h1);
             RF_STAMP(3, 0);
-            if (ASYNC) {
-                rf_bar_math();
-                rf_mbar_wait(&s_bar[0], (unsigned)t & 1u);
-            } else {
-                rf_cluster_arrive();
-                rf_cluster_wait();
-            }
+            rf_bar_math();                                    // hidden layer 1: own columns + the peers' columns
+            rf_mbar_wait(&s_bar[0], (unsigned)t & 1u);
             RF_STAMP(4, 0);
-            rf2_layer<false, ASYNC>(Hb1, p.ldh1, H1, W2s, Nc2, B2s, p.act[1], Hb2, p.ldh2, (int)crank * Nc2, Part, smem_base, crank, rf_t, 5,
-                                    bar_off_h2);
+            rf2_layer(Hb1, p.ldh1, H1, W2s, Nc2, B2s, p.act[1], Hb2, p.ldh2, (int)crank * Nc2, Part, smem_base, crank, rf_t,
+                      bar_off_h2);
             RF_STAMP(7, 0);
-            if (!ASYNC) {
-                rf_cluster_arrive();
-                rf_cluster_wait();
-            }
-            RF_STAMP(8, 0);
         } else {
             // ---- env warp h: everything of this step that does not depend on the action (arithmetic and Philox keys of
             // sample_one() / synth_env_block() in rollout.cu), concurrently with the layers
-            if (!ASYNC) rf_cluster_arrive();                  // barrier 1: nothing to publish
             RF_STAMP(16, 256);
             const int h = own;
             const long long ih = row0 + (int)crank * RF_OWN + h;
@@ -902,7 +436,7 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
             q = warp_sum(q);
             const bool h_done = (p.max_steps > 0) && (s_ep[h] + 1 >= p.max_steps);
             for (int d = lane; d < D; d += 32) {
-                float acc = 0.0f;
+                float acc = 0.0f;                              // WsT is [k][d]: conflict-free across lanes
 #pragma unroll 8
                 for (int k = 0; k < D; ++k) acc = fmaf(EWs[k * D + d], sh[k], acc);
                 const Philox4 r = philox4x32_10(p.env_seed ^ 0x5851F42D4C957F2Dull, ctr,
@@ -916,7 +450,7 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
                     Eq[2 * h + 1] = gz.y;
                 }
             }
-            if (!p.deterministic && lane < A) {
+            if (!p.deterministic && lane < A) {                // PPOAgent.act's N(0,1) draws: keys of sample_one()
                 const int j = lane;
                 const Philox4 r = philox4x32_10(p.agent_seed, ctr, ((unsigned long long)ih << 16) | (unsigned long long)(j >> 2));
                 const float2 z01 = box_muller(r.x, r.y), z23 = box_muller(r.z, r.w);
@@ -924,21 +458,13 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
                 Zn[h * A + j] = (c == 0) ? z01.x : (c == 1) ? z01.y : (c == 2) ? z23.x : z23.y;
             }
             RF_STAMP(17, 256);
-            if (!ASYNC) {
-                rf_cluster_wait();
-                rf_cluster_arrive();
-                rf_cluster_wait();
-            }
         }
-        if (ASYNC) {                                          // last hidden layer: own columns (block barrier) + the peers' columns
-            __syncthreads();
-            rf_mbar_wait(&s_bar[1], (unsigned)t & 1u);
-        }
-        // ---- head.  p.head_mode 1: warp w takes the k slice [w H2/16, (w+1) H2/16) for ALL 8 owned actors (lane = actor x 4 k
-        // sub-lanes), so the head weights are read from shared memory once per step instead of once per actor (the 2 x 8 KB
-        // per actor were 1 K cycles of the shared-memory pipe); the 16 slice sums meet in the (idle) Part buffer.
-        // head_mode 0: warps w and w + 8 take the two k halves of owned actor w & 7.
-        if (p.head_mode == 1) {
+        __syncthreads();                                      // last hidden layer: own columns + the peers' columns
+        rf_mbar_wait(&s_bar[1], (unsigned)t & 1u);
+        // ---- head: warp w takes the k slice [w H2/16, (w+1) H2/16) for ALL 8 owned actors (lane = actor x 4 k sub-lanes),
+        // so the head weights are read from shared memory once per step instead of once per actor (the 2 x 8 KB per actor
+        // were 1 K cycles of the shared-memory pipe); the 16 slice sums meet in the (idle) Part buffer.
+        {
             const int ks = H2 >> 4;                           // H2 % 16 == 0 (rf_plan)
             const int a8 = lane >> 2, ksub = lane & 3;
             const float* hrow = Hb2 + a8 * p.ldh2 + warp * ks;
@@ -978,49 +504,21 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
                 if (j0 < A) dst[j0] = t2[0];
                 if (j0 + 1 < A) dst[j0 + 1] = t2[1];
             }
-        } else {
-            const int half = warp >> 3;
-            const float* hrow = Hb2 + own * p.ldh2;
-            const int kh = H2 >> 1;
-            for (int n8 = 0; n8 < A; n8 += 8) {
-                float s8[8];
-#pragma unroll
-                for (int jj = 0; jj < 8; ++jj) s8[jj] = 0.0f;
-                const bool second = (n8 + 4 < ldwh);
-                for (int k = half * kh + lane; k < (half + 1) * kh; k += 32) {
-                    const float hv = hrow[k];
-                    const float* wr = Whs + k * ldwh + n8;
-                    const float4 w0 = *reinterpret_cast<const float4*>(wr);
-                    s8[0] = fmaf(hv, w0.x, s8[0]); s8[1] = fmaf(hv, w0.y, s8[1]);
-                    s8[2] = fmaf(hv, w0.z, s8[2]); s8[3] = fmaf(hv, w0.w, s8[3]);
-                    if (second) {
-                        const float4 w1 = *reinterpret_cast<const float4*>(wr + 4);
-                        s8[4] = fmaf(hv, w1.x, s8[4]); s8[5] = fmaf(hv, w1.y, s8[5]);
-                        s8[6] = fmaf(hv, w1.z, s8[6]); s8[7] = fmaf(hv, w1.w, s8[7]);
-                    }
-                }
-                const float v = rf_reduce8(s8, lane);
-                const int j = n8 + (((lane >> 4) & 1) << 2) + (((lane >> 3) & 1) << 1) + ((lane >> 2) & 1);
-                if ((lane & 3) == 0 && j < A) Hp[(half * RF_OWN + own) * A + j] = v;
-            }
         }
         RF_STAMP(9, 0);
         __syncthreads();
         RF_STAMP(10, 0);
         float rew = 0.0f, dn = 0.0f;
         int slot = SLOT_NONE;
+        // ---- owner warps: action, env step, bookkeeping -- same arithmetic, operand order and Philox keys as
+        // sample_one() / synth_env_block() of rollout.cu
         if (owner) {
             const int pos = s_pos[own];
             if (lane < A) {
                 const int j = lane;
-                float pre;
-                if (p.head_mode == 1) {
-                    pre = 0.0f;
+                float pre = 0.0f;
 #pragma unroll 4
-                    for (int w = 0; w < RF_THREADS / 32; ++w) pre += Part[(w * RF_OWN + own) * ldwh + j];    // fixed order
-                } else {
-                    pre = Hp[own * A + j] + Hp[(RF_OWN + own) * A + j];
-                }
+                for (int w = 0; w < RF_THREADS / 32; ++w) pre += Part[(w * RF_OWN + own) * ldwh + j];    // fixed order
                 RF_STAMP(19, 0);
                 const float mu = rf_act(pre + Bhs[j], p.act[2]);
                 const float sd = Sd[own * A + j];
@@ -1062,7 +560,7 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
                     p.reward[i_own] = rew;
                     p.done[i_own] = dn;
                 }
-                if (valid && pos + 1 == p.n_step) {
+                if (valid && pos + 1 == p.n_step) {            // this step completes a window -> next outbox entry
                     const int w = s_cnt[own];
                     if (w < p.Wout) {
                         slot = (int)(i_own * p.Wout + w);
@@ -1077,12 +575,14 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
             __syncwarp();
         }
         RF_STAMP(11, 0);
+        // ---- window staging (block-wide barriers inside: every warp calls; only owners do work)
         commit_actor(valid, (int)i_own, lane, 32, Nx + own * D, S + own * D, rew, dn, p.n_step, p.stride, D, A, s_pos + own,
                      slot, p.stage_obs, p.stage_act, p.stage_pd, p.stage_rew, p.stage_done, p.o_obs, p.o_act, p.o_pd, p.o_rew,
                      p.o_done);
         RF_STAMP(12, 0);
+        // ---- next observation -> z-filter -> every CTA's input tile
         if (owner) {
-            const int q4 = lane;
+            const int q4 = lane;                            // D / 4 <= 32 float4 per row
             if (q4 < (D >> 2)) {
                 float4 v = *reinterpret_cast<const float4*>(S + own * D + q4 * 4);
                 if (i_own >= p.N) v = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -1098,23 +598,17 @@ __global__ void __cluster_dims__(RF_CS, 1, 1) __launch_bounds__(RF_THREADS, 1)
                 float* qx = X0 + m_own * p.ldx0 + q4 * 4;
                 *reinterpret_cast<float4*>(qx) = v;
                 const unsigned off = rf_smem_u32(qx) - smem_base;
-                if (ASYNC) {
-                    if (!final_step) {
+                if (!final_step) {
 #pragma unroll
-                        for (int c = 0; c < RF_CS - 1; ++c) rf_st_async_v4(peer_base[c] + off, v, peer_base[c] + bar_off_x0);
-                    }
-                } else {
-#pragma unroll
-                    for (int c = 0; c < RF_CS - 1; ++c) rf_st_cluster_v4(peer_base[c] + off, v);
+                    for (int c = 0; c < RF_CS - 1; ++c) rf_st_async_v4(peer_base[c] + off, v, peer_base[c] + bar_off_x0);
                 }
             }
         }
         RF_STAMP(13, 0);
-        if (!ASYNC) cluster.sync();
-        RF_STAMP(14, 0);
     }
-    if (ASYNC) cluster.sync();                                // nobody leaves while a peer may still address its shared memory
+    cluster.sync();                                           // nobody leaves while a peer may still address its shared memory
 
+    // ---- write the per-actor control state back
     if (valid) {
         for (int d = lane; d < D; d += 32) p.state[i_own * D + d] = S[own * D + d];
         if (lane == 0) {
@@ -1220,11 +714,15 @@ bool rf_plan(const sb200_mlp* net, int D, int A, RfParams* p, size_t* smem_bytes
     const int oB = take(Nc1 + Nc2 + ldwh);
     const int ldx0 = D + 4, ldh1 = H1 + 4, ldh2 = H2 + 4;
     const int oX0 = take(RF_ROWS * ldx0), oH1 = take(RF_ROWS * ldh1), oH2 = take(RF_OWN * ldh2);
-    const int oPart = take(4LL * RF_ROWS * (Nc1 > Nc2 ? Nc1 : Nc2));
+    // k-split partial tiles of a hidden layer [4][32][max(Nc1, Nc2)] | the head's slice sums [16 warps][8][ldwh]
+    const int oPart = take(std::max(4LL * RF_ROWS * std::max(Nc1, Nc2), (long long)(RF_THREADS / 32) * RF_OWN * ldwh));
     const int oZf = take(2 * D), oEnv = take((long long)D * D + A * D);
-    const int oS = take(RF_OWN * D), oNext = take(RF_OWN * D), oAct = take(6 * RF_OWN * A);
+    const int oS = take(RF_OWN * D), oNext = take(RF_OWN * D), oAct = take(3 * RF_OWN * A);
     const int oPre = take(3 * RF_OWN * D + 2 * RF_OWN);
     if ((size_t)off * sizeof(float) > 224 * 1024) return false;
+    // each per-step hand-off counts the bytes a CTA receives from its 3 peers on one mbarrier, whose transaction count
+    // must stay below 2^20: hidden layer 1 (32 rows x Nc1), last hidden layer (8 rows x Nc2), next input tile (8 rows x D)
+    if (3LL * 4 * std::max({RF_ROWS * Nc1, RF_OWN * Nc2, RF_OWN * D}) >= (1 << 20)) return false;
     if (p != nullptr) {
         p->oW1 = oW1; p->oW2 = oW2; p->oWh = oWh; p->oB = oB; p->oX0 = oX0; p->oH1 = oH1; p->oH2 = oH2; p->oPart = oPart;
         p->oZf = oZf; p->oEnv = oEnv; p->oS = oS; p->oNext = oNext; p->oAct = oAct; p->oPre = oPre;
@@ -1238,10 +736,7 @@ bool rf_plan(const sb200_mlp* net, int D, int A, RfParams* p, size_t* smem_bytes
 }  // namespace
 
 int sb200_rollout_fused_init() {
-    SB200_CUDA(cudaFuncSetAttribute(ppo_rollout_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024));
-    SB200_CUDA(cudaFuncSetAttribute(ppo_rollout_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024));
-    SB200_CUDA(cudaFuncSetAttribute(ppo_rollout2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024));
-    SB200_CUDA(cudaFuncSetAttribute(ppo_rollout2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024));
+    SB200_CUDA(cudaFuncSetAttribute(ppo_rollout2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024));
     return SB200_OK;
 }
 
@@ -1316,24 +811,7 @@ extern "C" int sb200_ppo_rollout_f32(const sb200_ppo_rollout* a, void* stream) {
     p.T = a->T;
     p.step_ctr = (const unsigned long long*)a->step_counter;
     const long long clusters = ((long long)a->N + RF_ROWS - 1) / RF_ROWS;
-    // packed fma.rn.f32x2 in the hidden layers (default; bit-identical results, fewer issue slots: 1.764 -> 1.696 ms per
-    // 128-step chunk of 1024 actors).  SB200_RF_FFMA2=0 selects the scalar-FFMA instantiation.
-    static const int f2 = [] { const char* e = getenv("SB200_RF_FFMA2"); return e ? atoi(e) : 1; }();
-    // v2 (warp-specialised env warps, 8x4 register tiles) is the default; SB200_RF_V2=0 selects the v1 kernel
-    static const int v2 = [] { const char* e = getenv("SB200_RF_V2"); return e ? atoi(e) : 1; }();
-    static const int l1_direct = [] { const char* e = getenv("SB200_RF_L1DIRECT"); return e ? atoi(e) : 1; }();
-    p.l1_direct = (l1_direct && RF_ROWS == 4 * RF_OWN) ? 1 : 0;
-    static const int head_mode = [] { const char* e = getenv("SB200_RF_HEAD"); return e ? atoi(e) : 1; }();
-    // the slice sums need 16 warps x 8 actors x ldw[2] floats of the Part buffer (4 x 32 x max(Nc1, Nc2))
-    p.head_mode = (head_mode == 1 && 16 * RF_OWN * a->net->ldw[2] <= 4 * RF_ROWS * std::max(a->net->dims[1], a->net->dims[2]) / RF_CS) ? 1 : 0;
-    // default: mbarrier-signalled st.async hand-offs instead of the three cluster barriers per step (1.47 -> 1.38 ms per
-    // 128-step chunk of 1024 actors, same results bit for bit); SB200_RF_ASYNC=0 selects the barrier.cluster variant
-    static const int rf_async = [] { const char* e = getenv("SB200_RF_ASYNC"); return e ? atoi(e) : 1; }();
-    if (v2 && rf_async && a->D % 4 == 0 && (3u * RF_ROWS * (unsigned)(a->net->dims[1] / RF_CS) * 4u) < (1u << 20))
-        ppo_rollout2_kernel<true><<<(unsigned)(clusters * RF_CS), RF_THREADS, smem, (cudaStream_t)stream>>>(p);
-    else if (v2) ppo_rollout2_kernel<false><<<(unsigned)(clusters * RF_CS), RF_THREADS, smem, (cudaStream_t)stream>>>(p);
-    else if (f2) ppo_rollout_kernel<true><<<(unsigned)(clusters * RF_CS), RF_THREADS, smem, (cudaStream_t)stream>>>(p);
-    else ppo_rollout_kernel<false><<<(unsigned)(clusters * RF_CS), RF_THREADS, smem, (cudaStream_t)stream>>>(p);
+    ppo_rollout2_kernel<<<(unsigned)(clusters * RF_CS), RF_THREADS, smem, (cudaStream_t)stream>>>(p);
     return sb200_launch_status();
 }
 

@@ -361,14 +361,14 @@ def test_fused_rollout_launches_match_unfused(n, stride, cap_extra):
         assert torch.equal(f[k], u[k]), k
 
 
-def _rollout_pair(n, stride, cap_extra, zero_head, T, N=50, D=12, A=3):
+def _rollout_pair(n, stride, cap_extra, zero_head, T, actor_h=(48, 32), A=3, N=50, D=12):
     """Run the same chunk through the persistent rollout kernel and through the per-step launch sequence."""
     from surreal_b200.agent import PPOAgent
     from surreal_b200.replay import FIFOReplay
     from surreal_b200.env import SyntheticEnv
     out = []
     for persistent in (True, False):
-        lc, ec, sc = ppo_configs(D=D, A=A, actor_h=(48, 32), critic_h=(48, 32), n_step=n, stride=stride, B=8,
+        lc, ec, sc = ppo_configs(D=D, A=A, actor_h=actor_h, critic_h=(48, 32), n_step=n, stride=stride, B=8,
                                  memory_size=N + cap_extra)
         ec.num_envs = N
         R = FIFOReplay(lc, ec, sc)
@@ -401,12 +401,16 @@ def _rollout_pair(n, stride, cap_extra, zero_head, T, N=50, D=12, A=3):
     return out
 
 
-@pytest.mark.parametrize('n,stride,cap_extra', [(8, 8, 40), (6, 4, 40), (4, 4, -30), (5, 2, 100)])
-def test_persistent_rollout_matches_per_step_bitwise(n, stride, cap_extra):
+# 96x64-A32: a policy whose head's k-slice sums need more of the kernel's partial-sum buffer than its hidden layers do
+@pytest.mark.parametrize('n,stride,cap_extra,actor_h,A', [
+    pytest.param(8, 8, 40, (48, 32), 3, id='8-8-40'), pytest.param(6, 4, 40, (48, 32), 3, id='6-4-40'),
+    pytest.param(4, 4, -30, (48, 32), 3, id='4-4--30'), pytest.param(5, 2, 100, (48, 32), 3, id='5-2-100'),
+    pytest.param(8, 8, 40, (96, 64), 32, id='8-8-40-96x64-A32')])
+def test_persistent_rollout_matches_per_step_bitwise(n, stride, cap_extra, actor_h, A):
     """One persistent launch per chunk vs T x (forward, sample, env+commit): with a zero policy head both paths
     produce mean == 0 exactly, so sampling, env dynamics, window staging (overlapping windows, episode ends),
     outbox -> FIFO ordering in (step, actor) order and drop-oldest must agree bit for bit."""
-    p, s = _rollout_pair(n, stride, cap_extra, zero_head=True, T=29)
+    p, s = _rollout_pair(n, stride, cap_extra, zero_head=True, T=29, actor_h=actor_h, A=A)
     assert p['state'] == s['state'] and p['ctr'] == s['ctr'] == 29
     assert p['state']['total_in'] > 0 and (cap_extra > 0 or p['state']['dropped'] > 0)
     for k in ['pos', 'ep', 'env_state', 'act', 'pd', 'rew', 'done', 'obs_next', 'r_obs', 'r_act', 'r_pd', 'r_rew',
@@ -416,16 +420,17 @@ def test_persistent_rollout_matches_per_step_bitwise(n, stride, cap_extra):
 
 def test_persistent_rollout_policy_forward_close():
     """Same comparison with a live policy head: the cluster FFMA forward and the per-step tensor-core forward agree
-    to fp32 rounding, so trajectories stay within a small tolerance and every discrete quantity is identical."""
-    p, s = _rollout_pair(8, 8, 40, zero_head=False, T=16)
-    assert p['state'] == s['state'] and torch.equal(p['pos'], s['pos']) and torch.equal(p['ep'], s['ep'])
-    assert torch.equal(p['r_done'], s['r_done'])
-    A = 3
-    d0 = (p['r_pd'][:, 0, :A] - s['r_pd'][:, 0, :A]).abs().max()           # first step: identical inputs
-    assert float(d0) <= 1e-5, float(d0)
-    assert float(p['r_pd'][:, 0, :A].abs().max()) > 0.05                       # ... and a non-trivial policy output
-    for k in ['r_obs', 'r_act', 'r_pd', 'r_rew', 'env_state']:
-        assert float((p[k] - s[k]).abs().max()) <= 2e-3, (k, float((p[k] - s[k]).abs().max()))
+    to fp32 rounding, so trajectories stay within a small tolerance and every discrete quantity is identical.  The
+    second policy has a head whose k-slice sums need more of the kernel's partial-sum buffer than its hidden layers do."""
+    for actor_h, A in (((48, 32), 3), ((96, 64), 32)):
+        p, s = _rollout_pair(8, 8, 40, zero_head=False, T=16, actor_h=actor_h, A=A)
+        assert p['state'] == s['state'] and torch.equal(p['pos'], s['pos']) and torch.equal(p['ep'], s['ep'])
+        assert torch.equal(p['r_done'], s['r_done'])
+        d0 = (p['r_pd'][:, 0, :A] - s['r_pd'][:, 0, :A]).abs().max()           # first step: identical inputs
+        assert float(d0) <= 1e-5, (actor_h, float(d0))
+        assert float(p['r_pd'][:, 0, :A].abs().max()) > 0.05                       # ... and a non-trivial policy output
+        for k in ['r_obs', 'r_act', 'r_pd', 'r_rew', 'env_state']:
+            assert float((p[k] - s[k]).abs().max()) <= 2e-3, (actor_h, k, float((p[k] - s[k]).abs().max()))
 
 
 class NumpyScriptEnv:

@@ -6,7 +6,7 @@ mkdir -p gpurun_out
 SB200_CUDA_GRAPH=0 timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none -c 4000 --csv \
     --log-file gpurun_out/launches.csv python bench.py --steps 1 --warmup 3 --lite --sequential > gpurun_out/launches_bench.log 2>&1
 echo "launch list rc=$?"
-timeout 600 ncu --set full --clock-control none --import-source on -k regex:ppo_rollout2?_kernel -s 2 -c 1 \
+timeout 600 ncu --set full --clock-control none --import-source on -k ppo_rollout2_kernel -s 2 -c 1 \
     -o gpurun_out/prof_rollout -f python tools/prof_rollout.py 128 1 > gpurun_out/prof_rollout.log 2>&1
 echo "rollout capture rc=$?"
 timeout 300 ncu --set full --clock-control none --import-source on -k regex:mlp3_tc5 -s 2 -c 1 -f -o gpurun_out/prof_tc5 \

@@ -16,9 +16,10 @@ sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, 'tests'))
 OUT = os.path.join(ROOT, 'tools', '_trace')
 LIB = os.path.join(OUT, 'libsurreal_b200_trace.so')
-NAMES = {0: 'step top', 1: 'L1 fma done', 2: 'L1 sync', 3: 'L1 reduce+push', 4: 'cluster.sync 1', 5: 'L2 fma done', 6: 'L2 sync',
-         7: 'L2 reduce+push', 8: 'cluster.sync 2', 9: 'head (owner warp)', 10: 'phase-1 sync', 11: 'phase 2 (sample+env)',
-         12: 'commit_actor', 13: 'x0 push', 14: 'cluster.sync 3'}
+# (stamp id, phase that ends at it) in the order math warp 0 of a CTA passes them in one step; stamp 0 is the step top
+PHASES = [(18, 'input tile wait'), (3, 'L1 fma + push'), (4, 'L1 mbarrier wait'), (5, 'L2 fma'), (6, 'L2 sync'),
+          (7, 'L2 reduce + push'), (9, 'L2 wait + head slices'), (10, 'head sync'), (19, 'slice sums'),
+          (20, 'mean/sample/stores'), (21, 'env finalize'), (11, 'bookkeeping'), (12, 'commit_actor'), (13, 'x0 push')]
 
 
 def build():
@@ -65,19 +66,17 @@ def main():
     L.sb200_debug_rf_trace.argtypes = [C.c_void_p]
     assert L.sb200_debug_rf_trace(tr.ctypes.data_as(C.c_void_p)) == 0
     for cta in range(4):
-        print('CTA %d (cycles since step top; delta)' % cta)
+        print('CTA %d (cycles per phase, median over steps)' % cta)
         d = tr[cta]
-        per = np.zeros(15)
-        for i in range(1, 15):
-            per[i] = np.median(d[:, i] - d[:, i - 1])
+        prev, total = 0, 0.0
+        for i, name in PHASES:
+            c = np.median(d[:, i] - d[:, prev])
+            print('   %-24s %7.0f' % (name, c))
+            total += c
+            prev = i
         step = np.median(d[1:, 0] - d[:-1, 0])
-        for i in range(1, 15):
-            print('   %-24s %7.0f' % (NAMES[i], per[i]))
-        print('   %-24s %7.0f   (step period %0.f)' % ('sum', per.sum(), step))
-        print('   helper warp: start +%0.f after cluster.sync 2, busy %0.f' % (np.median(d[:, 16] - d[:, 8]), np.median(d[:, 17] - d[:, 16])))
-        if d[:, 18].any():
-            print('   v2 detail: input-tile wait ends +%0.f after step top; phase 2: slice sums %0.f | mean/sample/stores %0.f | env finalize %0.f | bookkeeping %0.f'
-                  % (np.median(d[1:, 18] - d[1:, 0]), np.median(d[:, 19] - d[:, 10]), np.median(d[:, 20] - d[:, 19]), np.median(d[:, 21] - d[:, 20]), np.median(d[:, 11] - d[:, 21])))
+        print('   %-24s %7.0f   (step period %0.f)' % ('sum', total, step))
+        print('   env warp: starts %+.0f from step top, busy %.0f' % (np.median(d[:, 16] - d[:, 0]), np.median(d[:, 17] - d[:, 16])))
 
 
 if __name__ == '__main__':
