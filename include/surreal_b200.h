@@ -141,12 +141,27 @@ int sb200_conv_backward_dw_f32(int layer, const void* x, int in_u8, const float*
                                double in_scale, float* slab_w, float* slab_b, int64_t slab_stride, int splits, void* stream);
 int sb200_conv_backward_dx_f32(int layer, const float* dy, const float* Wk, const float* act, int64_t frames, int CIN, int H,
                                int W, float* dx, void* stream);
+/* Conv layer 1 forward / weight gradient on uint8 frames that sit `row_bytes` apart (>= CIN*H*W) instead of back to back:
+ * the stem reads frames in place from wider records (the mixed pixel + low-dim observation rows).  With row_bytes = CIN*H*W
+ * these are exactly sb200_conv_forward_f32 / sb200_conv_backward_dw_f32 for layer 1 with in_u8 = 1. */
+int sb200_conv1_forward_u8_strided(const void* x, int64_t row_bytes, int64_t frames, int CIN, int H, int W, const float* Wk,
+                                   const float* bias, double in_scale, float* y, void* stream);
+int sb200_conv1_backward_dw_u8_strided(const void* x, int64_t row_bytes, const float* dy, int64_t frames, int CIN, int H, int W,
+                                       double in_scale, float* slab_w, float* slab_b, int64_t slab_stride, int splits,
+                                       void* stream);
 
 /* One step of the device-resident synthetic PIXEL env (SURVEY §8d cfg 4: uint8 frames of uniform random bytes, reward
  * -mean(a^2) + 0.1 N(0,1), done at the episode cap): state = the frames the actors observe next, obs_next = true successors. */
 int sb200_synth_pixel_env_step_u8(void* state, const float* action, int N, int64_t frame_bytes, int A, int max_steps,
                                   int* ep_step, uint64_t seed, const uint64_t* step_counter, void* obs_next, float* reward,
                                   float* done, void* stream);
+
+/* One step of the device-resident synthetic MIXED env: packed observation rows [N][row_words] = frame (frame_words 32-bit
+ * words of uint8 pixels, as synth_pixel_env) | D low-dim floats (dynamics, reward and done as synth_env) | zero padding.
+ * state = the rows the actors observe next, obs_next = true successors (same layout).  Ws / Wa in synth_env's layout. */
+int sb200_synth_mixed_env_step_f32(float* state, const float* action, const float* Ws, const float* Wa, int N, int D, int A,
+                                   int frame_words, int64_t row_words, int max_steps, int* ep_step, uint64_t seed,
+                                   const uint64_t* step_counter, float* obs_next, float* reward, float* done, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * One-shot all-reduce over NVLink peer memory (csrc/peer_allreduce.cu) for the small exchanges of the data-parallel

@@ -94,6 +94,7 @@ def _declare(lib):
         'sb200_mlp_tc5_workspace_bytes': (S, [C.POINTER(Mlp)]),
         'sb200_mlp_forward_tc5_f32': (I, [C.POINTER(Mlp), C.POINTER(ZFilter), C.POINTER(Rows), P, L, P, P]),
         'sb200_synth_pixel_env_step_u8': (I, [P, P, I, L, I, I, P, C.c_uint64, P, P, P, P, P]),
+        'sb200_synth_mixed_env_step_f32': (I, [P, P, P, P, I, I, I, I, L, I, P, C.c_uint64, P, P, P, P, P]),
         'sb200_par_buffer_bytes': (S, [L]),
         'sb200_par_alloc': (I, [L, C.POINTER(C.c_void_p), P]),
         'sb200_par_open': (I, [P, C.POINTER(C.c_void_p)]),
@@ -111,6 +112,8 @@ def _declare(lib):
         'sb200_conv_forward_f32': (I, [I, P, I, L, I, I, I, P, P, D, P, P]),
         'sb200_conv_backward_dw_f32': (I, [I, P, I, P, L, I, I, I, D, P, P, L, I, P]),
         'sb200_conv_backward_dx_f32': (I, [I, P, P, P, L, I, I, I, P, P]),
+        'sb200_conv1_forward_u8_strided': (I, [P, L, L, I, I, I, P, P, D, P, P]),
+        'sb200_conv1_backward_dw_u8_strided': (I, [P, L, P, L, I, I, I, D, P, P, L, I, P]),
         'sb200_mlp_pack_floats': (S, [C.POINTER(Mlp)]),
         'sb200_mlp_pack_tf32': (I, [C.POINTER(Mlp), P, P]),
         'sb200_mlp_forward_packed_f32': (I, [C.POINTER(Mlp), P, C.POINTER(ZFilter), C.POINTER(Rows), P, L, P]),

@@ -174,7 +174,11 @@ class Agent(metaclass=U.AutoInitializeMeta):
             raise ValueError('only the device-resident synthetic env ships with surreal_b200 (env_name "synthetic"); '
                              'gym / dm_control / robosuite adapters are out of scope -- pass your own env to '
                              'main_setup(env)')
-        from ..utils import obs_is_pixel
+        from ..utils import obs_is_pixel, obs_is_mixed
+        if obs_is_mixed(ec.obs_spec):
+            from ..env import SyntheticMixedEnv
+            return SyntheticMixedEnv(self.num_envs, ec.obs_spec, ec.action_spec.dim[0], ec.limit_episode_length,
+                                     seed=int(ec.seed) if 'seed' in ec else 0)
         if obs_is_pixel(ec.obs_spec):
             from ..env import SyntheticPixelEnv
             return SyntheticPixelEnv(self.num_envs, tuple(ec.obs_spec['pixel']['camera0']), ec.action_spec.dim[0],

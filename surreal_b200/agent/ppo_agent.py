@@ -69,6 +69,8 @@ class PPOAgent(Agent):
         """-> action (eval) or (action, [onetime_infos, [pd]]) in training, like ppo_agent.py:151-154.
         Device observations give device results; numpy in, numpy out."""
         N, A, D = self.num_envs, self.action_dim, self.model.low_dim
+        if self.model.mixed:
+            return self._act_mixed(obs, eps)
         if self.model.cnn_stem is not None:
             return self._act_pixel(obs, eps)
         if self.model.rnn_stem is not None:
@@ -248,6 +250,73 @@ class PPOAgent(Agent):
             self._stem_bufs = stem.buffers(N)
         feat = stem.forward(fr, self._stem_bufs)
         ops.mlp_forward(m.actor, feat, out=self._mean)
+        det = self.agent_mode in ['eval_deterministic', 'eval_deterministic_local']
+        env = self.env
+        staged = self.agent_mode == 'training' and isinstance(env, ExpSenderWrapperMultiStepMovingWindowWithInfo)
+        counter = env.step_counter if (env is not None and hasattr(env, 'step_counter')) else self._counter
+        eps_dev = None
+        if eps is not None:
+            eps_dev = torch.as_tensor(np.asarray(eps, dtype=np.float32).reshape(N, A)).to(self.device)
+        if staged and counter is not self._counter and env.fuse_launches:
+            fifo_state, dest = env.slot_assignment_args()
+            check(_lib.lib().sb200_ppo_sample_assign_f32(
+                _p(self._mean), A, _p(m.log_var), _p(self._log_noise), _p(eps_dev), N, A, int(det), self.seed,
+                _p(counter), _p(self._action), _p(self._pd), _p(env.stage_pos), _p(env.stage_act), _p(env.stage_pd),
+                env.n_step, _p(fifo_state), _p(dest), ops._stream()), 'sb200_ppo_sample_assign_f32')
+        else:
+            check(_lib.lib().sb200_ppo_sample_f32(
+                _p(self._mean), A, _p(m.log_var), _p(self._log_noise), _p(eps_dev), N, A, int(det), self.seed,
+                _p(counter), _p(self._action), _p(self._pd), _p(env.stage_pos) if staged else None,
+                _p(env.stage_act) if staged else None, _p(env.stage_pd) if staged else None,
+                env.n_step if staged else 1, ops._stream()), 'sb200_ppo_sample_f32')
+        if not staged and counter is self._counter:
+            self._counter += 1
+        if host:
+            if self._out_pin is None:
+                self._out_pin = (torch.empty(N, A, dtype=torch.float32, pin_memory=True),
+                                 torch.empty(N, 2 * A, dtype=torch.float32, pin_memory=True))
+            self._out_pin[0].copy_(self._action, non_blocking=True)
+            self._out_pin[1].copy_(self._pd, non_blocking=True)
+            torch.cuda.current_stream().synchronize()
+            action, pd = self._out_pin[0].numpy().astype(np.float64), self._out_pin[1].numpy().copy()
+        else:
+            action, pd = self._action, self._pd
+        if self.agent_mode != 'training':
+            return action
+        if self.env_config.sleep_time:
+            time.sleep(self.env_config.sleep_time)
+        return action, [[], [pd]]
+
+    def _act_mixed(self, obs, eps=None):
+        """act() on mixed observations (a camera frame + low-dim inputs): CNN stem on the frames -> actor head on
+        cat(zfilter(low_dim), features) (ppo_net.py:262-275) -> sampling kernel.  Both parts are read in place from the
+        packed observation rows (utils.obs_layout): the device env's own rows, or a host dict packed into a pinned row."""
+        from ..utils import obs_flat, obs_layout, pack_obs_rows
+        N, A = self.num_envs, self.action_dim
+        m, stem = self.model, self.model.cnn_stem
+        if getattr(self, '_layout', None) is None:
+            self._layout = obs_layout(self.obs_spec)
+            self._stem_bufs = stem.buffers(N)
+        lay = self._layout
+        W = lay['width']
+        host = not isinstance(obs['pixel']['camera0'], torch.Tensor)
+        if host:
+            if self._obs_pin is None:
+                self._obs_pin = torch.zeros(N, W, dtype=torch.float32, pin_memory=True)
+                self._rows_dev = torch.zeros(N, W, dtype=torch.float32, device=self.device)
+            pack_obs_rows(obs, lay, out=self._obs_pin.numpy())
+            self._rows_dev.copy_(self._obs_pin, non_blocking=True)
+            rows = self._rows_dev
+        else:
+            rows = obs_flat(obs, self.obs_spec)
+        feat = stem.forward(rows, self._stem_bufs, rows=N, row_bytes=4 * W)
+        ops.mlp_forward(m.actor, rows[:, lay['low_dim_off']:], zf_stats=m.z_stats, zf_eps=m.z_eps, aux=feat, rows=N, ldx=W,
+                        out=self._mean)
+        return self._sample(eps, host)
+
+    def _sample(self, eps, host):
+        """Sampling kernel on self._mean (+ staging of action / pd rows in training), then the act() return value."""
+        N, A, m = self.num_envs, self.action_dim, self.model
         det = self.agent_mode in ['eval_deterministic', 'eval_deterministic_local']
         env = self.env
         staged = self.agent_mode == 'training' and isinstance(env, ExpSenderWrapperMultiStepMovingWindowWithInfo)

@@ -32,7 +32,7 @@ template <int KS, int ST> __host__ __device__ inline int row_pitch(int W) { retu
 template <int KS, int ST, int COUT, typename IN_T>
 __global__ void __launch_bounds__(CT) conv_fwd_kernel(const IN_T* __restrict__ x, int frames, int CIN, int H, int W,
                                                       const float* __restrict__ Wk, const float* __restrict__ bias,
-                                                      float in_scale, float* __restrict__ y) {
+                                                      float in_scale, float* __restrict__ y, long long fsz) {
     extern __shared__ __align__(16) float sm[];
     const int HO = (H - KS) / ST + 1, WO = (W - KS) / ST + 1;
     const int Wp = row_pitch<KS, ST>(W);
@@ -48,7 +48,6 @@ __global__ void __launch_bounds__(CT) conv_fwd_kernel(const IN_T* __restrict__ x
     constexpr int SPAN = 3 * ST + KS;
     const int groups = (WO + 3) / 4;
     const int items = HO * groups * CQ;
-    const long long fsz = (long long)CIN * H * W;
     for (int f = blockIdx.x; f < frames; f += gridDim.x) {
         const IN_T* xf = x + (long long)f * fsz;
         for (int i = tid; i < CIN * H * W; i += CT) {
@@ -107,14 +106,13 @@ __global__ void __launch_bounds__(CT) conv_fwd_kernel(const IN_T* __restrict__ x
 template <int KS, int ST, int COUT, typename IN_T>
 __global__ void __launch_bounds__(CT) conv_bwd_dw_kernel(const IN_T* __restrict__ x, const float* __restrict__ dy, int frames,
                                                          int CIN, int H, int W, float in_scale, float* __restrict__ slab_w,
-                                                         float* __restrict__ slab_b, long long slab_stride) {
+                                                         float* __restrict__ slab_b, long long slab_stride, long long fsz) {
     extern __shared__ __align__(16) float sm[];
     const int HO = (H - KS) / ST + 1, WO = (W - KS) / ST + 1;
     const int taps = CIN * KS * KS, npos = HO * WO, npos4 = ru4(npos);
     float* xs = sm;                          // [CIN][H][W]
     float* ds = sm + ru4(CIN * H * W);       // [npos][COUT] (position-major: one LDS.128 broadcast per 4 channels)
     const int tid = threadIdx.x;
-    const long long fsz = (long long)CIN * H * W;
     float* out_w = slab_w + (long long)blockIdx.x * slab_stride;
     float* out_b = slab_b + (long long)blockIdx.x * slab_stride;
     (void)npos4;
@@ -215,22 +213,22 @@ constexpr size_t STEM_SMEM_MAX = 200 * 1024;
 
 template <int KS, int ST, int COUT, typename IN_T>
 int launch_fwd(const void* x, int frames, int CIN, int H, int W, const float* Wk, const float* bias, float in_scale, float* y,
-               cudaStream_t st) {
+               cudaStream_t st, long long fsz) {
     const size_t smem = ((size_t)CIN * KS * KS * COUT + (size_t)CIN * H * row_pitch<KS, ST>(W)) * sizeof(float);
     if (smem > STEM_SMEM_MAX) return SB200_ERR_UNSUPPORTED;
     const int grid = frames < 148 * 4 ? frames : 148 * 4;
-    conv_fwd_kernel<KS, ST, COUT, IN_T><<<grid, CT, smem, st>>>((const IN_T*)x, frames, CIN, H, W, Wk, bias, in_scale, y);
+    conv_fwd_kernel<KS, ST, COUT, IN_T><<<grid, CT, smem, st>>>((const IN_T*)x, frames, CIN, H, W, Wk, bias, in_scale, y, fsz);
     return sb200_launch_status();
 }
 
 template <int KS, int ST, int COUT, typename IN_T>
 int launch_dw(const void* x, const float* dy, int frames, int CIN, int H, int W, float in_scale, float* slab_w, float* slab_b,
-              long long slab_stride, int splits, cudaStream_t st) {
+              long long slab_stride, int splits, cudaStream_t st, long long fsz) {
     const int HO = (H - KS) / ST + 1, WO = (W - KS) / ST + 1;
     const size_t smem = ((size_t)ru4(CIN * H * W) + (size_t)HO * WO * COUT) * sizeof(float);
     if (smem > STEM_SMEM_MAX) return SB200_ERR_UNSUPPORTED;
     conv_bwd_dw_kernel<KS, ST, COUT, IN_T><<<splits, CT, smem, st>>>((const IN_T*)x, dy, frames, CIN, H, W, in_scale, slab_w, slab_b,
-                                                                     slab_stride);
+                                                                     slab_stride, fsz);
     return sb200_launch_status();
 }
 
@@ -255,15 +253,29 @@ extern "C" int sb200_conv_forward_f32(int layer, const void* x, int in_u8, int64
                                       const float* bias, double in_scale, float* y, void* stream) {
     SB200_REQUIRE(x && Wk && bias && y && frames >= 0 && CIN >= 1 && (layer == 1 || layer == 2));
     SB200_REQUIRE((((uintptr_t)Wk) & 15) == 0);
+    if (layer == 1 && in_u8) return sb200_conv1_forward_u8_strided(x, (int64_t)CIN * H * W, frames, CIN, H, W, Wk, bias, in_scale, y,
+                                                                   stream);
     if (frames == 0) return SB200_OK;
     cudaStream_t st = (cudaStream_t)stream;
+    const long long fsz = (long long)CIN * H * W;
     if (layer == 1) {
         SB200_REQUIRE(H >= 8 && W >= 8);
-        return in_u8 ? launch_fwd<8, 4, 16, unsigned char>(x, (int)frames, CIN, H, W, Wk, bias, (float)in_scale, y, st)
-                     : launch_fwd<8, 4, 16, float>(x, (int)frames, CIN, H, W, Wk, bias, (float)in_scale, y, st);
+        return launch_fwd<8, 4, 16, float>(x, (int)frames, CIN, H, W, Wk, bias, (float)in_scale, y, st, fsz);
     }
     SB200_REQUIRE(H >= 4 && W >= 4 && !in_u8);
-    return launch_fwd<4, 2, 32, float>(x, (int)frames, CIN, H, W, Wk, bias, (float)in_scale, y, st);
+    return launch_fwd<4, 2, 32, float>(x, (int)frames, CIN, H, W, Wk, bias, (float)in_scale, y, st, fsz);
+}
+
+// Conv layer 1 on uint8 frames that sit `row_bytes` apart (>= CIN*H*W): frames read in place from wider records, e.g. the
+// mixed pixel + low-dim observation rows of the staging / replay buffers (utils.obs_layout).
+extern "C" int sb200_conv1_forward_u8_strided(const void* x, int64_t row_bytes, int64_t frames, int CIN, int H, int W,
+                                              const float* Wk, const float* bias, double in_scale, float* y, void* stream) {
+    SB200_REQUIRE(x && Wk && bias && y && frames >= 0 && CIN >= 1);
+    SB200_REQUIRE((((uintptr_t)Wk) & 15) == 0 && row_bytes >= (int64_t)CIN * H * W);
+    if (frames == 0) return SB200_OK;
+    SB200_REQUIRE(H >= 8 && W >= 8);
+    return launch_fwd<8, 4, 16, unsigned char>(x, (int)frames, CIN, H, W, Wk, bias, (float)in_scale, y, (cudaStream_t)stream,
+                                               (long long)row_bytes);
 }
 
 // Partial weight / bias gradients of `frames` frames into `splits` slabs (slab s at slab_w + s*slab_stride, bias part at
@@ -272,13 +284,25 @@ extern "C" int sb200_conv_backward_dw_f32(int layer, const void* x, int in_u8, c
                                           int W, double in_scale, float* slab_w, float* slab_b, int64_t slab_stride, int splits,
                                           void* stream) {
     SB200_REQUIRE(x && dy && slab_w && slab_b && frames >= 1 && CIN >= 1 && splits >= 1 && (layer == 1 || layer == 2));
+    if (layer == 1 && in_u8)
+        return sb200_conv1_backward_dw_u8_strided(x, (int64_t)CIN * H * W, dy, frames, CIN, H, W, in_scale, slab_w, slab_b,
+                                                  slab_stride, splits, stream);
     cudaStream_t st = (cudaStream_t)stream;
+    const long long fsz = (long long)CIN * H * W;
     if (layer == 1)
-        return in_u8 ? launch_dw<8, 4, 16, unsigned char>(x, dy, (int)frames, CIN, H, W, (float)in_scale, slab_w, slab_b, slab_stride,
-                                                           splits, st)
-                     : launch_dw<8, 4, 16, float>(x, dy, (int)frames, CIN, H, W, (float)in_scale, slab_w, slab_b, slab_stride, splits, st);
+        return launch_dw<8, 4, 16, float>(x, dy, (int)frames, CIN, H, W, (float)in_scale, slab_w, slab_b, slab_stride, splits, st, fsz);
     SB200_REQUIRE(!in_u8);
-    return launch_dw<4, 2, 32, float>(x, dy, (int)frames, CIN, H, W, (float)in_scale, slab_w, slab_b, slab_stride, splits, st);
+    return launch_dw<4, 2, 32, float>(x, dy, (int)frames, CIN, H, W, (float)in_scale, slab_w, slab_b, slab_stride, splits, st, fsz);
+}
+
+// sb200_conv_backward_dw_f32 of layer 1 on uint8 frames `row_bytes` apart (see sb200_conv1_forward_u8_strided).
+extern "C" int sb200_conv1_backward_dw_u8_strided(const void* x, int64_t row_bytes, const float* dy, int64_t frames, int CIN,
+                                                  int H, int W, double in_scale, float* slab_w, float* slab_b, int64_t slab_stride,
+                                                  int splits, void* stream) {
+    SB200_REQUIRE(x && dy && slab_w && slab_b && frames >= 1 && CIN >= 1 && splits >= 1);
+    SB200_REQUIRE(row_bytes >= (int64_t)CIN * H * W);
+    return launch_dw<8, 4, 16, unsigned char>(x, dy, (int)frames, CIN, H, W, (float)in_scale, slab_w, slab_b, slab_stride, splits,
+                                              (cudaStream_t)stream, (long long)row_bytes);
 }
 
 // dx[frames][CIN][H][W] = relu'(act) * conv_transpose(dy, Wk) for layer 2 (its input is layer 1's post-ReLU output `act`).
@@ -348,4 +372,87 @@ extern "C" int sb200_synth_pixel_env_step_u8(void* state, const float* action, i
                                                                    (unsigned int*)obs_next, reward, done);
     synth_pixel_env_tick_kernel<<<(N + 255) / 256, 256, 0, (cudaStream_t)stream>>>(N, max_steps, ep_step);
     return sb200_launch_status(2);
+}
+
+// ------------------------------------------------------------------------------------------------------------------------
+// Synthetic MIXED environment: one camera frame plus a low-dim state per actor, written straight into the packed observation
+// rows the staging / replay kernels copy as opaque words (utils.obs_layout): row = [frame as frame_words 32-bit words |
+// D low-dim floats | zero padding to row_words].  The frame part is SyntheticPixelEnv's (same Philox keys: the same bytes for
+// the same seed and step), the low-dim part, the reward and done are SyntheticEnv's (s' = tanh(Ws s + Wa a) + 0.01 xi,
+// r = -|s|^2 / D + 0.1 xi', same keys and FMA order).  One CTA per actor, so the episode counter is updated in-kernel.
+namespace {
+__global__ void __launch_bounds__(256) synth_mixed_env_kernel(float* __restrict__ state, const float* __restrict__ action,
+                                                              const float* __restrict__ Ws, const float* __restrict__ Wa, int D,
+                                                              int A, int frame_words, long long row_words, int max_steps,
+                                                              int* __restrict__ ep_step, unsigned long long seed,
+                                                              const unsigned long long* __restrict__ step_ctr,
+                                                              float* __restrict__ obs_next, float* __restrict__ reward,
+                                                              float* __restrict__ done) {
+    extern __shared__ float sm[];            // [D] low-dim state, [A] action
+    __shared__ float s_q;
+    float* s_s = sm;
+    float* s_a = sm + D;
+    const int i = blockIdx.x, tid = threadIdx.x;
+    float* row = state + (long long)i * row_words;
+    float* nrow = obs_next + (long long)i * row_words;
+    for (int d = tid; d < D; d += 256) s_s[d] = row[frame_words + d];
+    for (int j = tid; j < A; j += 256) s_a[j] = action[(long long)i * A + j];
+    const unsigned long long ctr = (step_ctr != nullptr) ? *step_ctr : 0ull;
+    const int t = ep_step[i] + 1;
+    const bool dn = (max_steps > 0) && (t >= max_steps);
+    __syncthreads();
+    // frame: 4 words (16 pixels) per Philox draw
+    uint4* fr = reinterpret_cast<uint4*>(row);
+    uint4* nfr = reinterpret_cast<uint4*>(nrow);
+    for (int g = tid; g < frame_words / 4; g += 256) {
+        const Philox4 r = philox4x32_10(seed ^ 0x2545F4914F6CDD1Dull, ctr, ((unsigned long long)i << 24) | (unsigned long long)g);
+        uint4 nx = make_uint4(r.x, r.y, r.z, r.w);
+        nfr[g] = nx;
+        if (dn) {
+            const Philox4 z = philox4x32_10(seed ^ 0x9E3779B97F4A7C15ull, ctr, ((unsigned long long)i << 24) | (unsigned long long)g);
+            nx = make_uint4(z.x, z.y, z.z, z.w);
+        }
+        fr[g] = nx;
+    }
+    if (tid < 32) {
+        float q = 0.0f;
+        for (int d = tid; d < D; d += 32) q += s_s[d] * s_s[d];
+        q = warp_sum(q);
+        if (tid == 0) s_q = q;
+    }
+    __syncthreads();
+    for (int d = tid; d < D; d += 256) {
+        float acc = 0.0f;
+#pragma unroll 8
+        for (int k = 0; k < D; ++k) acc = fmaf(__ldg(Ws + (long long)k * D + d), s_s[k], acc);
+#pragma unroll 4
+        for (int k = 0; k < A; ++k) acc = fmaf(__ldg(Wa + (long long)k * D + d), s_a[k], acc);
+        const Philox4 r = philox4x32_10(seed ^ 0x5851F42D4C957F2Dull, ctr, ((unsigned long long)i << 20) | (unsigned long long)d);
+        const float2 g = box_muller(r.x, r.y);
+        const float nxt = tanhf(acc) + 0.01f * g.x;
+        nrow[frame_words + d] = nxt;
+        row[frame_words + d] = dn ? box_muller(r.z, r.w).x : nxt;
+        if (d == 0) {
+            reward[i] = -s_q / (float)D + 0.1f * g.y;
+            done[i] = dn ? 1.0f : 0.0f;
+        }
+    }
+    __syncthreads();                         // every thread has read ep_step[i]
+    if (tid == 0) ep_step[i] = dn ? 0 : t;
+}
+}  // namespace
+
+extern "C" int sb200_synth_mixed_env_step_f32(float* state, const float* action, const float* Ws, const float* Wa, int N, int D,
+                                              int A, int frame_words, int64_t row_words, int max_steps, int* ep_step, uint64_t seed,
+                                              const uint64_t* step_counter, float* obs_next, float* reward, float* done,
+                                              void* stream) {
+    SB200_REQUIRE(state && action && Ws && Wa && ep_step && obs_next && reward && done && N >= 1 && D >= 1 && A >= 1);
+    SB200_REQUIRE(frame_words >= 4 && frame_words % 4 == 0 && frame_words / 4 < (1 << 24) && D < (1 << 20));
+    SB200_REQUIRE(row_words >= (int64_t)frame_words + D && row_words % 4 == 0);
+    SB200_REQUIRE((((uintptr_t)state) & 15) == 0 && (((uintptr_t)obs_next) & 15) == 0);
+    SB200_REQUIRE((size_t)(D + A) * sizeof(float) <= 40 * 1024);
+    synth_mixed_env_kernel<<<N, 256, (size_t)(D + A) * sizeof(float), (cudaStream_t)stream>>>(
+        state, action, Ws, Wa, D, A, frame_words, (long long)row_words, max_steps, ep_step, (unsigned long long)seed,
+        (const unsigned long long*)step_counter, obs_next, reward, done);
+    return sb200_launch_status();
 }

@@ -13,7 +13,7 @@ from .. import _lib
 from .._lib import check
 from ..distributed import LocalHub
 from ..session import ConfigError
-from ..utils import obs_flat
+from ..utils import obs_flat, obs_is_mixed, obs_packed_dim
 
 
 def _p(t):
@@ -34,7 +34,11 @@ class _WrapperBase:
         if self.replay is None:
             raise RuntimeError('no replay registered for this session: construct the Replay before the agent '
                                'wraps its env (the ZeroMQ collector address of the reference is gone)')
-        self.N, self.D, self.A = env.N, env.D + int(obs_extra), env.A
+        # mixed observations (frame + low-dim): the rows are packed in the layout of utils.obs_layout, in this spec's key order
+        spec = env.observation_spec() if hasattr(env, 'observation_spec') else None
+        self.obs_spec = spec if (spec is not None and obs_is_mixed(spec)) else None
+        D = obs_packed_dim(self.obs_spec) if self.obs_spec is not None else env.D
+        self.N, self.D, self.A = env.N, D + int(obs_extra), env.A
         # extra trailing floats per observation row, filled by ``obs_augment(rows [N, env.D]) -> [N, D]`` (an RNN agent appends
         # its LSTM cells; utils.record_obs_dim)
         self.obs_extra, self.obs_augment = int(obs_extra), None
@@ -128,7 +132,7 @@ class ExpSenderWrapperMultiStepMovingWindowWithInfo(_WrapperBase):
     def reset(self):
         obs, info = self.env.reset()
         self.stage_pos.zero_()                                     # deque.clear() (exp_sender_wrapper.py:204-207)
-        o = obs_flat(obs)
+        o = obs_flat(obs, self.obs_spec)
         if self.host_env:
             d = self._h2d('obs', o, (self.N, self.D))
             self.stage_obs[:, 0].copy_(d)
@@ -172,8 +176,8 @@ class ExpSenderWrapperMultiStepMovingWindowWithInfo(_WrapperBase):
         if ready and hasattr(self.env, 'step_and_commit_window') and not self.obs_extra:
             return self.env.step_and_commit_window(a, self)        # env step + commit in ONE launch
         obs, reward, done, info = self.env.step(a)
-        o = obs_flat(obs)
-        on = obs_flat(info['obs_next']) if (isinstance(info, dict) and 'obs_next' in info) else o
+        o = obs_flat(obs, self.obs_spec)
+        on = obs_flat(info['obs_next'], self.obs_spec) if (isinstance(info, dict) and 'obs_next' in info) else o
         if self.host_env and self.obs_extra:
             raise NotImplementedError('RNN policy with a host env: stage the windows with replay.insert (onetime_infos) instead')
         if self.host_env:

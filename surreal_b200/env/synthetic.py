@@ -134,3 +134,73 @@ class SyntheticPixelEnv:
 
     def close(self):
         pass
+
+
+class SyntheticMixedEnv:
+    """Batched device-resident env with MIXED observations: one uint8 camera frame [C, H, W] and low-dim inputs per actor (the
+    robosuite observation, ppo_configs.py:111-114).  The frame follows SyntheticPixelEnv (fresh uniform random bytes every
+    step); the low-dim state follows SyntheticEnv (s' = tanh(Ws s + Wa a) + 0.01 xi); reward and done follow SyntheticEnv
+    (r = -|s|^2 / D + 0.1 xi', done at ``limit_episode_length``).  One kernel per step writes every actor's observation
+    straight into its packed record row (utils.obs_layout), which the window-staging kernels copy as opaque words; ``obs``
+    hands out views into those rows: ``'pixel'/'camera0'`` and one view per low-dim key."""
+    metadata = {}
+    graph_safe = True
+
+    def __init__(self, num_envs, obs_spec, action_dim=8, limit_episode_length=200, seed=0, device=None):
+        from ..utils import obs_layout, obs_is_mixed
+        if not torch.cuda.is_available():
+            raise RuntimeError('SyntheticMixedEnv is device-resident: a CUDA device is required')
+        if not obs_is_mixed(obs_spec):
+            raise ValueError('SyntheticMixedEnv needs a spec with a camera frame and low-dim inputs, got %s' % (obs_spec,))
+        self.device = torch.device(device if device is not None else ('cuda:%d' % torch.cuda.current_device()))
+        self.spec = {'pixel': {'camera0': tuple(obs_spec['pixel']['camera0'])},
+                     'low_dim': {k: tuple(v) for k, v in obs_spec['low_dim'].items()}}
+        self.layout = obs_layout(self.spec)
+        self.N, self.A = num_envs, action_dim
+        self.D = self.layout['width']                 # words per packed row: what the staging / replay records carry
+        self.low_dim = self.layout['low_dim']
+        self.max_steps = int(limit_episode_length)
+        self.seed = int(seed)
+        Dl = self.low_dim
+        g = torch.Generator().manual_seed(self.seed)  # as SyntheticEnv: the same seed gives the same low-dim dynamics
+        scale = 1.0 / (Dl ** 0.5)
+        self.Ws = (torch.randn(Dl, Dl, generator=g) * scale).to(self.device)
+        self.Wa = (torch.randn(Dl, action_dim, generator=g) * scale).to(self.device)
+        self.WsT, self.WaT = self.Ws.t().contiguous(), self.Wa.t().contiguous()
+        self._g = torch.Generator().manual_seed(self.seed + 1)
+        self.state = torch.zeros(num_envs, self.D, device=self.device)      # packed rows the actors observe next
+        self.obs_next = torch.zeros_like(self.state)                         # true successors (terminal where done)
+        self.ep_step = torch.zeros(num_envs, dtype=torch.int32, device=self.device)
+        self.reward = torch.zeros(num_envs, device=self.device)
+        self.done = torch.zeros(num_envs, device=self.device)
+        self.step_counter = torch.zeros(1, dtype=torch.int64, device=self.device)
+        from ..utils import mixed_obs_views
+        self._obs_state, self._obs_next = mixed_obs_views(self.state, self.layout), mixed_obs_views(self.obs_next, self.layout)
+
+    def observation_spec(self):
+        return self.spec
+
+    def action_spec(self):
+        return {'dim': (self.A,), 'type': 'continuous'}
+
+    def reset(self):
+        lay, N = self.layout, self.N
+        off = lay['low_dim_off']
+        frames = torch.randint(0, 256, (N, lay['frame_bytes']), generator=self._g, dtype=torch.uint8)
+        self.state.view(torch.uint8)[:, :lay['frame_bytes']].copy_(frames.to(self.device))
+        self.state[:, off:off + self.low_dim].copy_(torch.randn(N, self.low_dim, generator=self._g).to(self.device))
+        self.ep_step.zero_()
+        return self._obs_state, {}
+
+    def step(self, action):
+        if isinstance(action, tuple):
+            action = action[0]
+        lay = self.layout
+        check(_lib.lib().sb200_synth_mixed_env_step_f32(
+            _p(self.state), _p(action), _p(self.WsT), _p(self.WaT), self.N, self.low_dim, self.A, lay['frame_bytes'] // 4,
+            self.D, self.max_steps, _p(self.ep_step), self.seed + 7, _p(self.step_counter), _p(self.obs_next), _p(self.reward),
+            _p(self.done), _stream()), 'sb200_synth_mixed_env_step_f32')
+        return self._obs_state, self.reward, self.done, {'obs_next': self._obs_next}
+
+    def close(self):
+        pass

@@ -105,6 +105,10 @@ class PPOLearner(Learner):
 
         B, n, A = self.batch_size, self.n_step, self.action_dim
         self.pixel = self.model.cnn_stem is not None
+        # mixed observations (frame + low-dim): the pixel-mode launch chain with the low-dim columns as the heads' input and the
+        # CNN features as their layer-0 aux input; both read in place from the record rows (utils.obs_layout)
+        self.mixed = self.model.mixed
+        self.obs_layout = U.obs_layout(self.obs_spec) if self.mixed else None
         self.rnn = self.model.rnn_stem is not None
         self.obs_dim = self.model.low_dim                         # width of the low-dim features themselves
         # width of one observation in the batch buffers: the low-dim features (+ the actor's LSTM cells h | c in RNN mode,
@@ -116,7 +120,7 @@ class PPOLearner(Learner):
         M = B * self.eff_len                                      # rows the heads train on (ppo.py:518-537)
         self._rows = M
         dev = self.device
-        ig = 'linear' if self.rnn else self.pixel
+        ig = 'linear' if self.rnn else ('aux' if self.mixed else self.pixel)
         self.actor_optim = ops.MlpTrainer(self.model.actor, M, self.lr_actor,
                                           clip_mode=1 if self.clip_actor_gradient else 0,
                                           clip_value=self.actor_gradient_clip_value,
@@ -149,7 +153,8 @@ class PPOLearner(Learner):
             self._g_critic = torch.zeros(self.model.critic.size + stem.size, dtype=torch.float32, device=dev)
             self.actor_optim.grad = self._g_actor[:self.model.actor.size]
             self.critic_optim.grad = self._g_critic[:self.model.critic.size]
-            self._frames0 = torch.zeros(B, *stem_shape(stem), dtype=torch.uint8, device=dev)
+            # step-0 frames of every window, contiguous (pixel mode; mixed mode reads them in place)
+            self._frames0 = None if self.mixed else torch.zeros(B, *stem_shape(stem), dtype=torch.uint8, device=dev)
             self._stem_all = None                                 # activation buffers of the B*(n+1)-frame critic pass
             self._ref_stem_bufs = self.ref_target_model.cnn_stem.buffers(B)
 
@@ -279,6 +284,9 @@ class PPOLearner(Learner):
             own['obs_full'].copy_(full, non_blocking=True)
             nbytes += own['obs_full'].numel() * 4
             obs = None
+        elif self.mixed:
+            obs = None
+            nbytes += self._stage_mixed(get('obs'), get('obs_next'))
         elif self.pixel:
             obs = None
             fo, fn = get('obs')['pixel']['camera0'], get('obs_next')['pixel']['camera0']
@@ -327,6 +335,37 @@ class PPOLearner(Learner):
         self.last_h2d_bytes = nbytes
         return batch
 
+    def _stage_mixed(self, obs, obs_next):
+        """Mixed observation dicts (frames + low-dim keys, host or device) -> the record rows of obs_full.  Returns the bytes
+        sent host-to-device."""
+        B, n, lay = self.batch_size, self.n_step, self.obs_layout
+        full = self._own['obs_full']
+        if isinstance(obs['pixel']['camera0'], torch.Tensor):
+            for src, dst in ((obs, U.mixed_obs_views(full[:, :n], lay)), (obs_next, U.mixed_obs_views(full[:, n:], lay))):
+                d = dst['pixel']['camera0']
+                d.copy_(src['pixel']['camera0'].reshape(d.shape), non_blocking=True)
+                for k, _, _ in lay['keys']:
+                    dst['low_dim'][k].copy_(src['low_dim'][k].reshape(dst['low_dim'][k].shape), non_blocking=True)
+            return 0
+        if 'obs_full' not in self._pin:
+            self._pin['obs_full'] = torch.zeros(tuple(full.shape), dtype=torch.float32).pin_memory()
+        pf = self._pin['obs_full'].numpy()
+        pf[:, :n] = U.pack_obs_rows(obs, lay).reshape(B, n, -1)
+        pf[:, n:] = U.pack_obs_rows(obs_next, lay).reshape(B, 1, -1)
+        full.copy_(self._pin['obs_full'], non_blocking=True)
+        return full.numel() * 4
+
+    def _low_dim_cols(self):
+        """Mixed mode: the low-dim columns of the record rows (a view starting at the first one; callers pass rows / ldx)."""
+        return self._obs_full.view(-1)[self.obs_layout['low_dim_off']:]
+
+    def _mixed_stem(self, trainer=None, ref=False):
+        """Mixed mode: CNN features of the step-0 frame of every window, read in place from obs_full."""
+        rb = 4 * (self.n_step + 1) * self.low_dim
+        if trainer is not None:
+            return trainer.forward(self._obs_full, row_bytes=rb)
+        return self.ref_target_model.cnn_stem.forward(self._obs_full, self._ref_stem_bufs, rows=self.batch_size, row_bytes=rb)
+
     # ------------------------------------------------------------------------------------------------
     def _gae_and_return(self):
         """ppo.py:355-418 (MLP branch): critic over all B*(n+1) rows without materialising the cat, then GAE."""
@@ -341,6 +380,14 @@ class PPOLearner(Learner):
             h0, c0, ld = self._cells()
             h_all = m.rnn_stem.forward(self._xf_all, h0, c0, ld, B, n + 1, self._rnn_all)
             ops.mlp_forward(m.critic, h_all, out=self._values)
+        elif self.mixed:
+            # all B*(n+1) frames through the shared stem in place, then the critic head on (low-dim | features)
+            if self._stem_all is None:
+                self._stem_all = m.cnn_stem.buffers(rows)
+            D = self.low_dim
+            feat = m.cnn_stem.forward(self._obs_full, self._stem_all, rows=rows, row_bytes=4 * D)
+            ops.mlp_forward(m.critic, self._low_dim_cols(), zf_stats=m.z_stats, zf_eps=m.z_eps, aux=feat, rows=rows, ldx=D,
+                            out=self._values)
         elif self.pixel:
             # all B*(n+1) frames through the shared stem, then the critic head on the features (ppo.py:376-387, 5-D obs)
             stem = m.cnn_stem
@@ -439,6 +486,9 @@ class PPOLearner(Learner):
         acts, lda, pds, ldp = (self._act_it, A, self._pd_it, 2 * A) if self.rnn else (self._actions, n * A, self._pds, n * 2 * A)
         if self.rnn:
             mean = tr.forward(self.actor_rnn.forward(self._xf_eff, *self._cells())) if fresh else tr.out
+        elif self.mixed:
+            mean = tr.forward(self._low_dim_cols(), zf_stats=m.z_stats, zf_eps=m.z_eps, aux=self._mixed_stem(self.actor_stem),
+                              rows=B, ldx=(n + 1) * D) if fresh else tr.out
         elif self.pixel:
             mean = tr.forward(self.actor_stem.forward(self._frames0)) if fresh else tr.out
         else:
@@ -459,6 +509,12 @@ class PPOLearner(Learner):
             self.actor_rnn.backward(tr.dx0)
             joint_step(tr, self.actor_rnn, self._g_actor, norm_out=self._stats[S['GN_ACTOR']:S['GN_ACTOR'] + 1], stop_flag=stop)
             self._cur_mean = tr.forward(self.actor_rnn.forward(self._xf_eff, *self._cells()))
+        elif self.mixed:
+            from ..model.cnn_stem import joint_step
+            self.actor_stem.backward(tr.dx0)
+            joint_step(tr, self.actor_stem, self._g_actor, norm_out=self._stats[S['GN_ACTOR']:S['GN_ACTOR'] + 1], stop_flag=stop)
+            self._cur_mean = tr.forward(self._low_dim_cols(), zf_stats=m.z_stats, zf_eps=m.z_eps,
+                                        aux=self._mixed_stem(self.actor_stem), rows=B, ldx=(n + 1) * D)
         elif self.pixel:
             from ..model.cnn_stem import joint_step
             self.actor_stem.backward(tr.dx0)
@@ -493,6 +549,8 @@ class PPOLearner(Learner):
             raise NotImplementedError('reward filter + data parallel')
         if self.rnn:
             raise NotImplementedError('RNN mode + data parallel')
+        if self.mixed:
+            raise NotImplementedError('mixed pixel + low-dim observations + data parallel')
         stem_n = self.model.cnn_stem.size if self.pixel else 0
         peer_floats = max(self.model.actor.size, self.model.critic.size) + stem_n + 64
         self.dp = LearnerDP(group, peer_floats=peer_floats)
@@ -537,6 +595,9 @@ class PPOLearner(Learner):
         m, tr, st = self.model, self.critic_optim, ops._stream()
         if self.rnn:
             v = tr.forward(self.critic_rnn.forward(self._xf_eff, *self._cells()))
+        elif self.mixed:
+            v = tr.forward(self._low_dim_cols(), zf_stats=m.z_stats, zf_eps=m.z_eps, aux=self._mixed_stem(self.critic_stem),
+                           rows=B, ldx=(n + 1) * D)
         elif self.pixel:
             v = tr.forward(self.critic_stem.forward(self._frames0))
         else:
@@ -548,7 +609,7 @@ class PPOLearner(Learner):
             from ..model.cnn_stem import joint_step
             self.critic_rnn.backward(tr.dx0)
             joint_step(tr, self.critic_rnn, self._g_critic, norm_out=self._stats[S['GN_CRITIC']:S['GN_CRITIC'] + 1])
-        elif self.pixel:
+        elif self.pixel:                                          # pixel and mixed: the stem takes the features' gradient
             from ..model.cnn_stem import joint_step
             self.critic_stem.backward(tr.dx0)
             joint_step(tr, self.critic_stem, self._g_critic, norm_out=self._stats[S['GN_CRITIC']:S['GN_CRITIC'] + 1])
@@ -562,6 +623,9 @@ class PPOLearner(Learner):
         if self.rnn:
             h_ref = ref.rnn_stem.forward(self._xf_ref, *self._cells(), B, self.eff_len, self._rnn_ref)
             ops.mlp_forward(ref.actor, h_ref, out=self._ref_mean)
+        elif self.mixed:
+            ops.mlp_forward(ref.actor, self._low_dim_cols(), zf_stats=ref.z_stats, zf_eps=ref.z_eps, aux=self._mixed_stem(ref=True),
+                            rows=B, ldx=(n + 1) * D, out=self._ref_mean)
         elif self.pixel:
             # step-0 frames of every window, contiguous (ppo.py:527-537), then the reference policy on them
             fr = self._obs_full.view(torch.uint8).view(B, n + 1, -1)
@@ -590,6 +654,8 @@ class PPOLearner(Learner):
             # updates (ppo.py:578)
             if self.rnn:
                 ops.zfilter_update(self._xraw_eff, self._rows, self.obs_dim, self._xraw_eff.stride(0), m.z_stats)
+            elif self.mixed:
+                ops.zfilter_update(self._low_dim_cols(), B, self.obs_dim, (n + 1) * D, m.z_stats)
             elif self.dp is None:
                 ops.zfilter_update(self._obs_full, B, D, (n + 1) * D, m.z_stats)
             else:

@@ -88,15 +88,23 @@ class CNNStem:
         f = lambda *s: torch.empty(*s, dtype=torch.float32, device=self.device)  # noqa: E731
         return dict(a1=f(rows, self.C1, self.H1, self.W1), a2=f(rows, self.flat), feat=f(rows, self.d_out))
 
-    def forward(self, frames, bufs, params=None):
+    def forward(self, frames, bufs, params=None, rows=None, row_bytes=None):
         """frames: uint8 [rows, C, H, W] contiguous (raw 0..255; scaled by 1/255 inside, ppo_net.py:370) -> feat [rows, d_out].
+        With ``row_bytes``, ``frames`` is any CUDA tensor whose first byte is the first frame and ``rows`` frames sit
+        ``row_bytes`` apart (read in place from mixed observation records, utils.obs_layout).
         ``bufs`` (from ``buffers(rows)``) receives the intermediate activations a1 / a2 (needed by the backward pass)."""
-        assert frames.dtype == torch.uint8 and frames.is_cuda and frames.is_contiguous()
-        rows = frames.shape[0]
         L, st = _lib.lib(), ops._stream()
         P = self.params if params is None else params
-        check(L.sb200_conv_forward_f32(1, _p(frames), 1, rows, self.C, self.H, self.W, _p(self.seg('w1', P)), _p(self.seg('b1', P)),
-                                       1.0 / 255.0, _p(bufs['a1']), st), 'sb200_conv_forward_f32(1)')
+        if row_bytes is None:
+            assert frames.dtype == torch.uint8 and frames.is_cuda and frames.is_contiguous()
+            rows = frames.shape[0]
+            check(L.sb200_conv_forward_f32(1, _p(frames), 1, rows, self.C, self.H, self.W, _p(self.seg('w1', P)),
+                                           _p(self.seg('b1', P)), 1.0 / 255.0, _p(bufs['a1']), st), 'sb200_conv_forward_f32(1)')
+        else:
+            assert frames.is_cuda and row_bytes >= self.C * self.H * self.W
+            check(L.sb200_conv1_forward_u8_strided(_p(frames), int(row_bytes), rows, self.C, self.H, self.W, _p(self.seg('w1', P)),
+                                                   _p(self.seg('b1', P)), 1.0 / 255.0, _p(bufs['a1']), st),
+                  'sb200_conv1_forward_u8_strided')
         check(L.sb200_conv_forward_f32(2, _p(bufs['a1']), 0, rows, self.C1, self.H1, self.W1, _p(self.seg('w2', P)),
                                        _p(self.seg('b2', P)), 1.0, _p(bufs['a2']), st), 'sb200_conv_forward_f32(2)')
         ops.mlp_forward(self.fc, bufs['a2'], params=self.seg('fc', P), out=bufs['feat'])
@@ -118,10 +126,12 @@ class StemTrainer:
         self.d_a2 = z(M, stem.flat)                               # ... conv2's pre-activation
         self.d_a1 = z(M, stem.C1, stem.H1, stem.W1)               # ... conv1's pre-activation
         self.frames = None
+        self.row_bytes = None
 
-    def forward(self, frames):
-        self.frames = frames
-        return self.stem.forward(frames, self.bufs)
+    def forward(self, frames, row_bytes=None):
+        """``row_bytes``: the M frames are read in place, ``row_bytes`` apart (see CNNStem.forward)."""
+        self.frames, self.row_bytes = frames, row_bytes
+        return self.stem.forward(frames, self.bufs, rows=self.M, row_bytes=row_bytes)
 
     def backward(self, d_feat_pre):
         """``d_feat_pre`` [M, >= d_out]: gradient w.r.t. the Linear layer's PRE-activation (the head's input gradient already
@@ -144,9 +154,14 @@ class StemTrainer:
         check(L.sb200_conv_backward_dx_f32(2, _p(self.d_a2), _p(s.seg('w2')), _p(b['a1']), M, s.C1, s.H1, s.W1, _p(self.d_a1), st),
               'sb200_conv_backward_dx_f32')
         o_w1, o_b1 = s.off['w1'][0], s.off['b1'][0]
-        check(L.sb200_conv_backward_dw_f32(1, _p(self.frames), 1, _p(self.d_a1), M, s.C, s.H, s.W, 1.0 / 255.0,
-                                           C.c_void_p(base + 4 * o_w1), C.c_void_p(base + 4 * o_b1), s.size, self.splits, st),
-              'sb200_conv_backward_dw_f32(1)')
+        if self.row_bytes is None:
+            check(L.sb200_conv_backward_dw_f32(1, _p(self.frames), 1, _p(self.d_a1), M, s.C, s.H, s.W, 1.0 / 255.0,
+                                               C.c_void_p(base + 4 * o_w1), C.c_void_p(base + 4 * o_b1), s.size, self.splits, st),
+                  'sb200_conv_backward_dw_f32(1)')
+        else:
+            check(L.sb200_conv1_backward_dw_u8_strided(_p(self.frames), int(self.row_bytes), _p(self.d_a1), M, s.C, s.H, s.W,
+                                                       1.0 / 255.0, C.c_void_p(base + 4 * o_w1), C.c_void_p(base + 4 * o_b1),
+                                                       s.size, self.splits, st), 'sb200_conv1_backward_dw_u8_strided')
 
     def state_dict(self):
         return {'exp_avg': self.exp_avg.detach().clone(), 'exp_avg_sq': self.exp_avg_sq.detach().clone()}

@@ -26,7 +26,8 @@ def _default_linear_init(dims, seed_gen=None):
 
 class PPOModel:
     """Same constructor keywords as the reference's PPOModel (ppo_net.py:110-118).  The LSTM stem is a
-    'next' row of SURVEY §8f and raises here; the CNN stem (pixel input) is model/cnn_stem.py."""
+    'next' row of SURVEY §8f and raises here; the CNN stem (pixel input) is model/cnn_stem.py.  With pixel input AND
+    low-dim inputs (mixed observations) the heads' layer 0 takes the low-dim columns followed by the CNN features."""
 
     def __init__(self, obs_spec, action_dim, model_config, use_cuda=True, init_log_sig=0, use_z_filter=False,
                  if_pixel_input=False, rnn_config=None, device=None):
@@ -43,11 +44,11 @@ class PPOModel:
         if 'low_dim' in obs_spec:
             for key in obs_spec['low_dim']:
                 self.low_dim += obs_spec['low_dim'][key][0]
+        # mixed observations (a camera frame AND low-dim inputs): the heads see cat([zfilter(low_dim), cnn_features], -1)
+        # (ppo_net.py:262-275); here the features are the aux input of layer 0, next to the low-dim columns
+        self.mixed = bool(if_pixel_input and self.low_dim > 0)
         if if_pixel_input:
             # optional CNN stem feature extractor (ppo_net.py:136-140), shared by actor and critic
-            if self.low_dim > 0:
-                raise NotImplementedError('mixed low_dim + pixel observations (ppo_net.py:268-275 concatenates them) are not '
-                                          'supported: the HBM replay records carry one observation kind')
             from .cnn_stem import CNNStem
             self.cnn_stem = CNNStem(obs_spec['pixel']['camera0'], model_config.cnn_feature_dim, self.device)
         in_dim = self.low_dim + (model_config.cnn_feature_dim if if_pixel_input else 0)
@@ -61,10 +62,12 @@ class PPOModel:
         D, A = in_dim, action_dim
         ah, ch = list(model_config.actor_fc_hidden_sizes), list(model_config.critic_fc_hidden_sizes)
         R, T, N = ops.ACT_RELU, ops.ACT_TANH, ops.ACT_NONE
-        self.actor = ops.FlatNet([D] + ah + [A], [R] * len(ah) + [T], self.device, extra=A)
-        self.critic = ops.FlatNet([D] + ch + [1], [R] * len(ch) + [N], self.device)
-        self.actor.load_layers(_default_linear_init(self.actor.dims), extra=torch.zeros(A) + init_log_sig)
-        self.critic.load_layers(_default_linear_init(self.critic.dims))
+        aux = dict(aux_layer=0, aux_dim=model_config.cnn_feature_dim) if self.mixed else {}
+        Dx = self.low_dim if self.mixed else D
+        self.actor = ops.FlatNet([Dx] + ah + [A], [R] * len(ah) + [T], self.device, extra=A, **aux)
+        self.critic = ops.FlatNet([Dx] + ch + [1], [R] * len(ch) + [N], self.device, **aux)
+        self.actor.load_layers(_default_linear_init([D] + ah + [A]), extra=torch.zeros(A) + init_log_sig)
+        self.critic.load_layers(_default_linear_init([D] + ch + [1]))
         self.z_eps = 1e-5
         self.z_stats = None
         if use_z_filter:
@@ -167,8 +170,20 @@ class PPOModel:
             self._stem_bufs, self._stem_bufs_rows = self.cnn_stem.buffers(rows), rows
         return self.cnn_stem.forward(fr, self._stem_bufs)
 
+    def _mixed_inputs(self, obs):
+        """Mixed mode: (low-dim rows [rows, Dl], CNN features [rows, F]) of an observation dict."""
+        x = self._flat(obs)
+        return x.reshape(-1, x.shape[-1]).contiguous(), self._features(obs)
+
     def forward_actor(self, obs, cells=None, out_pd=None):
         """-> [rows, 2A] = cat(mean, std) (builders.py:114-132)."""
+        if self.mixed:
+            x2, feat = self._mixed_inputs(obs)
+            mean = ops.mlp_forward(self.actor, x2, zf_stats=self.z_stats, zf_eps=self.z_eps, aux=feat)
+            B, A = mean.shape[0], self.action_dim
+            pd = out_pd if out_pd is not None else torch.empty(B, 2 * A, dtype=torch.float32, device=self.device)
+            ops.make_pd(mean, self.log_var, B, A, pd)
+            return pd
         if self.cnn_stem is not None:
             x2 = self._features(obs)
             mean = ops.mlp_forward(self.actor, x2)
@@ -185,6 +200,9 @@ class PPOModel:
         return pd
 
     def forward_critic(self, obs, cells=None):
+        if self.mixed:
+            x2, feat = self._mixed_inputs(obs)
+            return ops.mlp_forward(self.critic, x2, zf_stats=self.z_stats, zf_eps=self.z_eps, aux=feat)
         if self.cnn_stem is not None:
             return ops.mlp_forward(self.critic, self._features(obs))
         x = self._flat(obs)

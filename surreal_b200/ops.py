@@ -307,7 +307,10 @@ class MlpTrainer:
         self._aux_pad = None
         # gradient w.r.t. the pre-activation of whatever produced the network input (times relu'(input)): the CNN stem's
         # Linear layer sits in front of the PPO heads in pixel mode
-        self.dx0 = z(M, _ru(net.dims[0], 4)) if input_grad else None
+        # 'aux': the gradient w.r.t. the aux input of layer 0 instead (times relu'(aux)): the CNN features next to the low-dim
+        # inputs of a mixed observation
+        dx0_w = net.aux_dim if input_grad == 'aux' else net.dims[0]
+        self.dx0 = z(M, _ru(dx0_w, 4)) if input_grad else None
         self.input_grad = input_grad            # True / 'relu': times relu'(input) (CNN stem's Linear+ReLU); 'linear': as is (LSTM output)
         self.overlap_dw = os.environ.get('SB200_OVERLAP_DW', '1') != '0'
         self._side = None
@@ -377,7 +380,13 @@ class MlpTrainer:
                     dw_layer(l, _stream())
             else:
                 dw_layer(l, _stream())
-        if self.dx0 is not None:
+        if self.input_grad == 'aux':
+            lay = net.layout[0]
+            w_aux = net.params.data_ptr() + 4 * (lay['w'] + net.dims[0] * lay['ldw'])
+            check(L.sb200_linear_bwd_dx_f32(_ptr(self.d[0]), self.d[0].stride(0), C.c_void_p(w_aux), lay['ldw'], _ptr(self.aux),
+                                            self.aux.stride(0), _ptr(self.dx0), self.dx0.stride(0), M, lay['N'], net.aux_dim,
+                                            _stream()), 'sb200_linear_bwd_dx_f32(aux input)')
+        elif self.dx0 is not None:
             lay = net.layout[0]
             check(L.sb200_linear_bwd_dx_f32(_ptr(self.d[0]), self.d[0].stride(0), C.c_void_p(net.params.data_ptr() + 4 * lay['w']),
                                             lay['ldw'], _ptr(None if self.input_grad == 'linear' else self.x_in), self.x_in.stride(0), _ptr(self.dx0), self.dx0.stride(0), M,

@@ -40,10 +40,12 @@ class FIFOReplay(Replay):
             raise RuntimeError('surreal_b200.FIFOReplay lives in HBM: a CUDA device is required')
         self.device = torch.device('cuda', torch.cuda.current_device())
         self.n_step = self.learner_config.algo.n_step
-        from ..utils import record_obs_dim, obs_packed_dim, obs_is_pixel
+        from ..utils import record_obs_dim, obs_packed_dim, obs_is_pixel, obs_is_mixed, obs_layout
         self.D = record_obs_dim(self.learner_config, self.env_config)   # pixel frames: opaque 32-bit words; RNN: + LSTM cells
         self.obs_dim = obs_packed_dim(self.env_config.obs_spec)
         self.pixel_shape = tuple(self.env_config.obs_spec['pixel']['camera0']) if obs_is_pixel(self.env_config.obs_spec) else None
+        # mixed observations: frame words + low-dim floats in one row (utils.obs_layout)
+        self.layout = obs_layout(self.env_config.obs_spec) if obs_is_mixed(self.env_config.obs_spec) else None
         self.A = self.env_config.action_spec.dim[0]
         self.capacity = self.memory_size + 3                    # "+ 3 for a gentle buffering" (fifo_replay.py:27)
         C_, n, D, A = self.capacity, self.n_step, self.D, self.A
@@ -81,7 +83,10 @@ class FIFOReplay(Replay):
         """``exp``: the dict ExpSenderWrapperMultiStepMovingWindowWithInfo.send emits
         (exp_sender_wrapper.py:244-264): obs [n dicts], obs_next, actions, rewards, dones, persistent_infos."""
         n, D, A = self.n_step, self.D, self.A
-        if self.pixel_shape is not None:       # uint8 frame -> the same bytes viewed as float32 words
+        if self.layout is not None:
+            from ..utils import pack_obs_rows
+            flat = lambda o: pack_obs_rows(o, self.layout).reshape(-1)  # noqa: E731
+        elif self.pixel_shape is not None:       # uint8 frame -> the same bytes viewed as float32 words
             flat = lambda o: np.ascontiguousarray(np.asarray(o['pixel']['camera0'], dtype=np.uint8)).reshape(-1).view(np.float32)  # noqa: E731
         else:
             flat = lambda o: np.concatenate([np.asarray(o['low_dim'][k], dtype=np.float32).reshape(-1)  # noqa: E731
@@ -137,6 +142,12 @@ class FIFOReplay(Replay):
         if self.check_underflow and int(self._status.item()) != 0:      # host sync; the engine polls
             raise IndexError('pop from a FIFO replay holding fewer than %d windows' % batch_size)   # len() instead
         obs_full = out['obs_full']
+        if self.layout is not None:
+            # views into the batch: uint8 frames [B, n(+1), C, H, W] and one [B, n(+1), width] view per low-dim key
+            from ..utils import mixed_obs_views
+            return {'obs': mixed_obs_views(obs_full[:, :n], self.layout), 'obs_next': mixed_obs_views(obs_full[:, n:], self.layout),
+                    'obs_full': obs_full, 'actions': out['actions'], 'rewards': out['rewards'], 'dones': out['dones'],
+                    'persistent_infos': [out['pd']], 'onetime_infos': None}
         if self.pixel_shape is not None:
             fr = obs_full.view(torch.uint8).view(batch_size, n + 1, *self.pixel_shape)
             return {'obs': {'pixel': {'camera0': fr[:, :n]}}, 'obs_next': {'pixel': {'camera0': fr[:, n:]}},

@@ -7,7 +7,11 @@ graph per chunk) followed by PPOLearner.learn() on the 256 windows (stem + criti
 that train the shared stem through both optimisers).  Under torchrun every rank runs its own 256 actors (weak scaling) and
 the learner is data-parallel.
 
-    python tools/bench_pixel.py [steps]          |   torchrun --nproc-per-node N tools/bench_pixel.py [steps]
+``--low-dim D`` adds a D-float low-dim input next to the frame (mixed observations, the robosuite spec of
+ppo_configs.py:111-114): the records carry frame + low-dim, the heads take cat(zfilter(low_dim), features) and the z-filter
+is on.  Single GPU only (the mixed learner has no data-parallel path).
+
+    python tools/bench_pixel.py [steps] [--low-dim D]   |   torchrun --nproc-per-node N tools/bench_pixel.py [steps]
 """
 import copy
 import json
@@ -21,8 +25,13 @@ import torch  # noqa: E402
 
 
 def main():
+    import argparse
     import torch.distributed as dist
-    steps = int(sys.argv[1]) if len(sys.argv) > 1 else 5
+    ap = argparse.ArgumentParser()
+    ap.add_argument('steps', type=int, nargs='?', default=5)
+    ap.add_argument('--low-dim', type=int, default=0, help='floats of low-dim input next to the frame (0: pixel only)')
+    args = ap.parse_args()
+    steps, Dl = args.steps, args.low_dim
     rank, world, local = int(os.environ.get('RANK', 0)), int(os.environ.get('WORLD_SIZE', 1)), int(os.environ.get('LOCAL_RANK', 0))
     torch.cuda.set_device(local)
     dev = torch.device('cuda', local)
@@ -47,6 +56,11 @@ def main():
     lc.replay.batch_size, lc.replay.memory_size = N, 2 * N
     lc.parameter_publish.exp_interval, lc.parameter_publish.min_publish_interval = N, 0.0
     make_synthetic_pixel_env_config(ec, N, SHAPE, A, seed=rank)
+    if Dl > 0:
+        if world > 1:
+            raise SystemExit('--low-dim: the mixed-observation learner runs on one GPU')
+        ec.obs_spec = {'low_dim': {'robot-state': (Dl,)}, 'pixel': {'camera0': SHAPE}}
+        lc.algo.use_z_filter = True
     ec.limit_episode_length = 2 * T
     sc.agent.fetch_parameter_interval = T
     la = SurrealDefaultLauncher(PPOAgent, PPOLearner, FIFOReplay, sc, ec, lc)
@@ -79,8 +93,10 @@ def main():
         total = float(t.item())
     if rank == 0:
         frame = SHAPE[0] * SHAPE[1] * SHAPE[2]
-        print(json.dumps({'workload': 'PPO synthetic pixel 84x84x4 uint8, 256 actors per GPU x horizon 128, CNN 16k8s4-32k4s2-FC256 + 2x256 heads '
-                                      '(BASELINE configs[3])', 'n_gpus': world, 'steps': steps,
+        mixed = ' + %d low-dim floats (z-filtered)' % Dl if Dl else ''
+        print(json.dumps({'workload': 'PPO synthetic pixel 84x84x4 uint8%s, 256 actors per GPU x horizon 128, CNN 16k8s4-32k4s2-FC256 + '
+                                      '2x256 heads (BASELINE configs[3])' % mixed, 'low_dim': Dl, 'n_gpus': world, 'steps': steps,
+                          'gpu': torch.cuda.get_device_name(dev),
                           'env_steps_per_s': N * T * steps * world / (total / 1e3), 'ms_per_step': total / steps,
                           'rollout_ms': roll, 'learn_ms': learn, 'frame_bytes_in_hbm': frame, 'algorithmic_frame_bytes': 28224,
                           'frames_through_stem_per_step': N * T + N * (T + 1) + 21 * N * 3,
